@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: SV-DGCNN clouds/sec (binary, ModelNet40 head, N=1024, k=20).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one forward of the hot path over one batch of B=32 synthetic clouds per GPU
 (BASELINE.json configs[1]).  Multi-GPU (launched by torchrun, one rank per GPU) shards by cloud
@@ -16,6 +16,10 @@ the reference's own models/*.py, stock PyTorch on the host cores, all threads) o
 Extra keys of our line: `gpu_eager_reference` (the same reference modules on cuda: stock eager fp32),
 `extra.cfg3` / `extra.cfg4` / `extra.cfg5` (BASELINE.json configs[2] / configs[3] / three points of configs[4]'s sweep, batch-sharded over the ranks: strong
 scaling, cfg4 with the all-gather of the per-point logits inside the timed region).
+`--dump-outputs DIR` writes what the last timed step returned (rank 0): DIR/logits.npy, float32 (B, 40), and with
+several ranks DIR/logits_gathered.npy, the all-gathered (world * B, 40); with `--impl reference`, DIR/logits.npy
+(n, 40) of that arm's last timed forward over its n clouds.  Clouds and checkpoint are seeded, so two builds of the
+project run on identical inputs and their dumps can be compared array for array.
 """
 import argparse
 import contextlib
@@ -126,7 +130,7 @@ def cpu_port_throughput(n_clouds, reps=1):
         dt = time.perf_counter() - t0
         best = dt if best is None else min(best, dt)
     assert np.isfinite(y).all()
-    return n_clouds / best, best
+    return n_clouds / best, best, y
 
 
 def dbg(msg):
@@ -179,7 +183,7 @@ def reference_cpu_throughput(n_clouds, steps, warmup, budget_s=240.0):
             if i >= warmup:
                 per_step.append(dt)
     assert bool(torch.isfinite(y).all())
-    return n, per_step
+    return n, per_step, y.numpy()
 
 
 def run_reference(args):
@@ -190,16 +194,24 @@ def run_reference(args):
     cores = os.cpu_count()
     from oracle import reference
     if reference.available():
-        n, per_step = reference_cpu_throughput(B_PER_GPU, args.steps, args.warmup)
+        n, per_step, y = reference_cpu_throughput(B_PER_GPU, args.steps, args.warmup)
         kind = "reference"
         what = ("%d clouds per step; unmodified reference forward (oracle/_ref/models, models/sv_dgcnn_cls.py:46-82), "
                 "stock PyTorch CPU, torch.set_num_threads(%d)" % (n, cores))
     else:   # oracle/_ref not staged on this box: fall back to the C + OpenMP restatement (still a CPU arm)
-        v0, _ = cpu_port_throughput(4)
+        v0, _, _ = cpu_port_throughput(4)
         n = int(min(64, max(4, round(2.0 * v0 / 4) * 4)))
-        per_step = [cpu_port_throughput(n)[1] for _ in range(args.warmup + args.steps)][args.warmup:]
+        per_step = []
+        for i in range(args.warmup + args.steps):
+            _, dt, y = cpu_port_throughput(n)
+            if i >= args.warmup:
+                per_step.append(dt)
         kind = "port"
         what = "%d clouds per step, oracle C port with OpenMP (oracle/_ref missing)" % n
+    if args.dump_outputs:                 # the logits of the last timed forward: (n, 40) for its n clouds
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "logits.npy"), np.asarray(y, dtype=np.float32))
     ms = 1e3 * sum(per_step) / len(per_step)
     value = n / (ms / 1e3)
     out = {
@@ -309,7 +321,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip extra.cfg3 / extra.cfg4 / gpu_eager_reference")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the logits of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 0)
     if args.impl == "reference":
         return run_reference(args)
@@ -398,8 +413,23 @@ def main():
         barrier()
         # ---- device-resident throughput (graph replay of the public call) ----
         dbg("warm-up done")
-        ms = timed(lambda: step(x_dev), args.steps)
+        last = {"steps": 0}
+
+        def graph_step():
+            last["logits"] = step(x_dev)
+            last["steps"] += 1
+        ms = timed(graph_step, args.steps)
+        timed_steps = last["steps"]
         dbg("graph steps timed")
+        if args.dump_outputs and rank == 0:
+            # the replay's output buffer (and `gathered`) are overwritten by every later call: save them now
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            dump = {"logits": last["logits"]}
+            if world > 1:
+                dump["logits_gathered"] = gathered
+            for name, t in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), t.float().cpu().numpy())
         # ---- the same K steps eagerly, with the dominant C-ABI calls bracketed by CUDA events on their
         #      launch stream (events cannot bracket kernels inside a graph replay) ----
         from svnet_b200 import fused as sv_fused
@@ -547,13 +577,13 @@ def main():
     if not args.no_cpu_baseline and world == 1:             # rank 0 at N = 1 only (bench contract)
         use_all_host_threads()
         from oracle import reference
-        v, dt = cpu_port_throughput(4)                      # probe, then a sample worth ~5 s of CPU work
+        v, dt, _ = cpu_port_throughput(4)                   # probe, then a sample worth ~5 s of CPU work
         n_cpu = int(min(128, max(4, round(5.0 * v / 4) * 4)))
-        v, dt = cpu_port_throughput(n_cpu)
+        v, dt, _ = cpu_port_throughput(n_cpu)
         port = {"value": v, "unit": "clouds/s", "kind": "port",
                 "sample": "%d clouds of the same workload (N=1024, k=20), oracle C port with OpenMP, %.1f s" % (n_cpu, dt)}
         if reference.available():
-            n_ref, per_step = reference_cpu_throughput(B_PER_GPU, 2, 1, budget_s=45.0)
+            n_ref, per_step, _ = reference_cpu_throughput(B_PER_GPU, 2, 1, budget_s=45.0)
             best = min(per_step)
             cpu = {"value": n_ref / best, "unit": "clouds/s", "cores": os.cpu_count(), "kind": "reference",
                    "sample": "%d clouds of the same workload per forward, best of %d after 1 warm-up (%.1f s each); unmodified "
@@ -563,7 +593,7 @@ def main():
             cpu = dict(port, cores=os.cpu_count())
 
     out = {
-        "metric": METRIC, "value": world * B / (ms * 1e-3), "unit": "clouds/s", "n_gpus": world, "steps": args.steps,
+        "metric": METRIC, "value": world * B / (ms * 1e-3), "unit": "clouds/s", "n_gpus": world, "steps": timed_steps,
         "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32 (+u32 XNOR/popcount for the binarised linears; exact bf16x3 tcgen05 filter in front of the fp32 kNN)", "data": "synthetic",
         "config": bench_config(world),
@@ -574,7 +604,7 @@ def main():
                 "h2d_bytes_per_step": x_host.numel() * 4, "d2h_bytes_per_step": y_host.numel() * 4},
         # kernels of libsvnet_b200.so inside the timed region: K replays of the captured forward (four
         # sub-batches); the eager single-stream pass used for the per-kernel events launches `eager` per step
-        "gpu_launches": kernels_per_replay * args.steps,
+        "gpu_launches": kernels_per_replay * timed_steps,
         "gpu_launches_per_step": {"graph_replay": kernels_per_replay, "eager_single_stream": launches},
         "roofline": roofline,
         "cpu_baseline": cpu,

@@ -68,13 +68,17 @@ def knn_agreement(feat_bcn, ref_idx, our_idx, tol=2e-5):
             "worst_rel_gap": worst, "unexplained_rows": unexplained, "tol": tol}
 
 
-def build_pair(kind, k, binary, ncls, seed, dev):
+def build_ours(kind, k, binary, ncls, seed, dev):
     import svnet_b200 as sv
-    ref = reference.load()
     ours = quiet(getattr(sv, kind), make_args(k=k, binary=binary), ncls)
     sd = synthetic_state_dict(ours.state_dict(), seed=seed)
     ours.load_state_dict(sd)
-    ours = ours.to(dev).eval()
+    return ours.to(dev).eval(), sd
+
+
+def build_pair(kind, k, binary, ncls, seed, dev):
+    ref = reference.load()
+    ours, sd = build_ours(kind, k, binary, ncls, seed, dev)
     rnet = quiet(getattr(ref, kind), make_args(k=k, binary=binary), ncls)
     rnet.load_state_dict(sd)
     rnet = rnet.to(dev).eval()
@@ -84,20 +88,120 @@ def build_pair(kind, k, binary, ncls, seed, dev):
 MODEL_FILE = {"SV_DGCNN_CLS": "sv_dgcnn_cls", "SV_DGCNN_PSEG": "sv_dgcnn_partseg"}
 
 
-def measure(kind="SV_DGCNN_CLS", B=4, N=1024, k=20, binary=True, ncls=40, seed=1002, dev="cuda"):
+SIGN_OF = ["conv2.linear1", "conv3.linear1", "conv4.linear1"]
+
+
+class Record:
+    """What measure() compares against, recorded from one forward: the layer inputs of the kNN calls (B, C, N),
+    the kNN indices, the pooled per-point (s, v) of the four edge layers, for binary models the sign planes
+    sign(u + beta) and |u + beta| of conv2-4's linear1, and the logits."""
+
+    def __init__(self, knn_in, idx, pools, signs, logits):
+        self.knn_in, self.idx, self.pools, self.signs, self.logits = knn_in, idx, pools, signs, logits
+
+
+def reference_record(rnet, kind, x, extra, binary):
+    """The unmodified reference forward (oracle/_ref), hooked by reference.Recorder."""
+    modfile = reference.submodule(MODEL_FILE[kind])
+    with torch.no_grad(), reference.Recorder(modfile, rnet, SIGN_OF if binary else []) as rec:
+        y_ref = rnet(x, *extra)
+    return Record(rec.knn_in[:4], rec.idx[:4], rec.pools[:4], rec.signs, y_ref)
+
+
+def oracle_record(sd, kind, k, binary, x, extra, dev):
+    """The same record from the CPU oracle (oracle/svnet_oracle.c, the reference restated function by function and
+    pinned to the reference's own outputs by tests/test_oracle_golden.py), for where the reference's model code is not
+    staged.  The oracle is deterministic: tests/golden/refparity_*.npz hold samples of its record at these shapes
+    (tests/golden/make_golden_refparity.py), and pin_to_golden() checks every run against them."""
+    from oracle import svnet_oracle as orc
+    xn = x.cpu().numpy()
+    rec = {}
+    if kind == "SV_DGCNN_PSEG":
+        y = orc.sv_dgcnn_pseg(sd, xn, extra[0].cpu().numpy(), k, rec=rec)
+    else:
+        y = orc.sv_dgcnn_cls(sd, xn, k, rec=rec)
+    P = orc.Params(sd)
+    B, N = xn.shape[0], xn.shape[2]
+    knn_in, signs = [x], {}
+    for li in range(1, 4):
+        s, v = rec["pools"][li - 1]
+        knn_in.append(torch.from_numpy(np.concatenate([s, v.reshape(B, N, -1)], axis=-1)).to(dev).transpose(1, 2))
+        if binary:
+            cname = "conv%d" % (li + 1)
+            s_e, v_e = orc.graph_feature_sv(s, v, rec["idx"][li])
+            u = np.concatenate([s_e, orc.p_v2s(P.sub(cname + ".v2s"), v_e)], axis=-1)
+            beta = P.get(cname + ".linear1.beta").reshape(-1)
+            signs[cname + ".linear1"] = (torch.from_numpy(orc.sign_plane(u, beta)).to(dev),
+                                         torch.from_numpy(np.abs(u + beta)).to(dev))
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+    return Record(knn_in, [t(i) for i in rec["idx"]], [(t(s), t(v)) for s, v in rec["pools"]], signs, t(y))
+
+
+# the BASELINE.json shapes of the parity test (batch cut to keep the CPU side short)
+CASES = {
+    "cfg2": dict(kind="SV_DGCNN_CLS", B=4, N=1024, k=20, binary=True, ncls=40, seed=1002),
+    "cfg3": dict(kind="SV_DGCNN_CLS", B=4, N=1024, k=20, binary=False, ncls=15, seed=1003),
+    "cfg4": dict(kind="SV_DGCNN_PSEG", B=2, N=2048, k=40, binary=True, ncls=50, seed=1004),
+}
+GOLDEN_ROWS = 24       # sampled points (kNN rows, pooled features, per-point logits) and edge rows (sign planes)
+
+
+def golden_samples(r, seed=0):
+    """Fixed, seeded sample of a Record as numpy arrays (what tests/golden/refparity_*.npz store)."""
+    B, N = r.idx[0].shape[:2]
+    g = np.random.default_rng(seed)
+    pts = np.sort(g.choice(B * N, GOLDEN_ROWS, replace=False))
+    out = {"points": pts}
+    for li in range(4):
+        out["idx%d" % li] = r.idx[li].reshape(B * N, -1)[pts].cpu().numpy().astype(np.int16)
+        s, v = r.pools[li]
+        out["pool%d_s" % li] = s.reshape(B * N, -1)[pts].cpu().numpy()
+        out["pool%d_v" % li] = v.reshape(B * N, 3, -1)[pts].cpu().numpy()
+    for name, (sign, _) in sorted(r.signs.items()):
+        K = sign.shape[-1]
+        edges = np.sort(g.choice(sign.numel() // K, GOLDEN_ROWS, replace=False))
+        out["edges|" + name] = edges
+        out["sign|" + name] = sign.reshape(-1, K)[edges].cpu().numpy()
+    y = r.logits
+    out["logits"] = (y.cpu().numpy() if y.dim() == 2 else
+                     y.permute(0, 2, 1).reshape(B * N, -1)[pts].cpu().numpy())   # part-seg: (B, parts, N)
+    return out
+
+
+def pin_to_golden(r, golden):
+    """The oracle's record equals the stored one on every sampled element: indices and sign planes exactly, floats to
+    a few ulps (the oracle's summation order is fixed; only the host's libm may differ)."""
+    got = golden_samples(r)
+    assert sorted(got) == sorted(k for k in golden.files if k != "config"), (sorted(got), golden.files)
+    for key, val in got.items():
+        want = golden[key]
+        assert val.shape == want.shape and val.dtype == want.dtype, key
+        if val.dtype.kind == "f":
+            assert np.allclose(val, want, rtol=1e-6, atol=1e-7), "oracle record differs from tests/golden at " + key
+        else:
+            assert np.array_equal(val, want), "oracle record differs from tests/golden at " + key
+
+
+def measure(kind="SV_DGCNN_CLS", B=4, N=1024, k=20, binary=True, ncls=40, seed=1002, dev="cuda", golden=None):
+    """golden=None: against the unmodified reference forward; else (an np.load of tests/golden/refparity_*.npz)
+    against the oracle's record, pinned to those samples."""
     import svnet_b200 as sv
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
-    ours, rnet, sd = build_pair(kind, k, binary, ncls, seed, dev)
     x = synthetic_clouds(B, N, seed).to(dev)
     extra = (one_hot_labels(B).to(dev),) if kind == "SV_DGCNN_PSEG" else ()
-    sign_of = ["conv2.linear1", "conv3.linear1", "conv4.linear1"] if binary else []
-    modfile = reference.submodule(MODEL_FILE[kind])
-    with torch.no_grad(), reference.Recorder(modfile, rnet, sign_of) as rec:
-        y_ref = rnet(x, *extra)
-    out = {"model": kind, "B": B, "N": N, "k": k, "binary": binary, "layers": []}
-    ridx = rec.idx[:4]
-    pools = rec.pools[:4]
+    if golden is None:
+        ours, rnet, sd = build_pair(kind, k, binary, ncls, seed, dev)
+        rec = reference_record(rnet, kind, x, extra, binary)
+    else:
+        (ours, sd), rnet = build_ours(kind, k, binary, ncls, seed, dev), None
+        rec = oracle_record(sd, kind, k, binary, x, extra, dev)
+        pin_to_golden(rec, golden)
+    y_ref = rec.logits
+    out = {"model": kind, "B": B, "N": N, "k": k, "binary": binary, "layers": [],
+           "against": "reference" if golden is None else "oracle"}
+    ridx = rec.idx
+    pools = rec.pools
     teacher = [(s.reshape(B * N, -1).contiguous(), v.reshape(B * N, 3, -1).contiguous()) for s, v in pools[:3]]
     got = {"teacher": teacher, "want_taps": True}
     forced = [i.to(torch.int32).contiguous() for i in ridx]

@@ -1,33 +1,27 @@
-"""GPU parity against the UNMODIFIED reference forward at the BASELINE.json shapes.
+"""GPU parity against the reference forward at the BASELINE.json shapes.
 
-The reference's model code is staged into oracle/_ref (git-ignored, ships with the snapshot) by
-oracle/make_ref.sh; here it runs on the same device and inputs as the CUDA path, and every kind of
-disagreement is counted and explained (tests/refparity.py).  Bars: north_star's correctness clause
-with SURVEY.md 7.3.1 / 7.3.2's account of where stock ATen and a fixed summation order may differ.
+Where the reference's model code is staged into oracle/_ref (git-ignored) by oracle/make_ref.sh, the UNMODIFIED
+reference runs on the same device and inputs as the CUDA path.  Elsewhere the same record comes from the CPU oracle
+(the reference restated in C, pinned to the reference's own outputs by tests/test_oracle_golden.py), checked against
+the samples of it stored in tests/golden/refparity_<cfg>.npz.  Every kind of disagreement is counted and explained
+(tests/refparity.py).  Bars: north_star's correctness clause with SURVEY.md 7.3.1 / 7.3.2's account of where stock
+ATen and a fixed summation order may differ.
 """
 import json
-import os
 
 import pytest
-import torch
 
 from oracle import reference
+from tests import refparity
+from tests.util import golden
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not reference.available(), reason="oracle/_ref not staged (sh oracle/make_ref.sh)")]
-
-CASES = {
-    "cfg2": dict(kind="SV_DGCNN_CLS", B=4, N=1024, k=20, binary=True, ncls=40, seed=1002),
-    "cfg3": dict(kind="SV_DGCNN_CLS", B=4, N=1024, k=20, binary=False, ncls=15, seed=1003),
-    "cfg4": dict(kind="SV_DGCNN_PSEG", B=2, N=2048, k=40, binary=True, ncls=50, seed=1004),
-}
+pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("cfg", ["cfg2", "cfg3", "cfg4"])
 def test_full_size_parity_with_reference_forward(cfg):
-    from tests import refparity
-    kw = CASES[cfg]
-    out, _ = refparity.measure(**kw)
+    kw = refparity.CASES[cfg]
+    out, _ = refparity.measure(**kw, golden=None if reference.available() else golden("refparity_" + cfg))
     print(cfg, json.dumps(out))
     for st in out["layers"]:
         # kNN: identical rows, or a differing row is a swap / boundary exchange between candidates whose

@@ -1,5 +1,7 @@
 """CPU: pin the oracle (oracle/svnet_oracle.{c,py}) against the golden fixtures produced by the
 unmodified reference (tests/golden/make_golden.py).  The reference has no tests of its own."""
+import json
+
 import numpy as np
 import pytest
 
@@ -143,3 +145,18 @@ def test_svblock_binary_sign_plane_matches_reference():
     so, vo = orc.svblock(P, (s, v))
     assert_close(so, g["svb_bin_so"], rtol=1e-5, atol=1e-5)
     assert_close(vo, g["svb_bin_vo"], rtol=1e-4, atol=1e-5)
+
+
+@pytest.mark.parametrize("cfg", ["cfg2", "cfg3", "cfg4"])
+def test_oracle_record_at_baseline_shapes_matches_golden(cfg):
+    """The oracle's record at the full-size parity test's shapes (tests/refparity.py: what the CUDA path is compared
+    against where the reference's model code is not staged) reproduces the samples stored in tests/golden."""
+    from tests import refparity
+    from svnet_b200.synthetic import one_hot_labels, synthetic_clouds
+    kw = refparity.CASES[cfg]
+    g = golden("refparity_" + cfg)
+    assert json.loads(str(g["config"])) == kw
+    _, sd = refparity.build_ours(kw["kind"], kw["k"], kw["binary"], kw["ncls"], kw["seed"], "cpu")
+    x = synthetic_clouds(kw["B"], kw["N"], kw["seed"])
+    extra = (one_hot_labels(kw["B"]),) if kw["kind"] == "SV_DGCNN_PSEG" else ()
+    refparity.pin_to_golden(refparity.oracle_record(sd, kw["kind"], kw["k"], kw["binary"], x, extra, "cpu"), g)

@@ -1,6 +1,6 @@
 import contextlib, io, os, sys
 import torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import svnet_b200 as sv
 from svnet_b200 import _native as nv, fused
 from svnet_b200.synthetic import make_args, synthetic_clouds, synthetic_state_dict
