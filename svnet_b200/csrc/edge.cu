@@ -389,8 +389,9 @@ extern "C" int svnet_svblock_edge_fwd(const svnet_edge_params* p, void* stream)
     if ((long)p->B * p->N == 0) return SVNET_OK;
     if (p->binary) {
         SV_REQUIRE(p->beta && p->W1b && p->scale1, "svnet_svblock_edge_fwd: binary layer needs beta/W1b/scale1");
-        // shapes of the SV-DGCNN models have compile-time specialisations (edge_fast.cu);
-        // SVNET_EDGE_GENERIC=1 forces the generic kernel (tests cover both)
+        // shapes of the SV-DGCNN models have compile-time specialisations (edge_fast.cu, edge_tc.cu);
+        // SVNET_EDGE_GENERIC=1 forces the generic kernel below (tests/test_gpu_edge_fp64.py runs it next to the
+        // specialised ones against a float64 restatement of the layer)
         const char* force = getenv("SVNET_EDGE_GENERIC");
         if (!(force && force[0] == '1')) {
             // tensor-core kernel when the caller supplied its packed weights and table scratch (edge_tc.cu)
@@ -402,6 +403,7 @@ extern "C" int svnet_svblock_edge_fwd(const svnet_edge_params* p, void* stream)
             if (h < 0) return h;
             if (h == 1) return SVNET_OK;
         }
+        SV_REQUIRE(p->PQ, "svnet_svblock_edge_fwd: the generic kernel needs the PQ table");
         return launch_edge<true>(p, sv_stream(stream));
     }
     SV_REQUIRE(p->Yab, "svnet_svblock_edge_fwd: fp layer needs Yab");

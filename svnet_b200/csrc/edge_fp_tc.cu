@@ -438,6 +438,10 @@ bool ftc_covered(int cs, int cv, int co, int cvo, int k)
     if (off && off[0] == '0') return false;
     const char* tc = getenv("SVNET_TCGEN05");          // the per-point table comes from the tcgen05 vector linear
     if (tc && tc[0] == '0') return false;
+    const char* fp = getenv("SVNET_VLINEAR_FP_TC");    // ... with full-precision weights: its three-plane path
+    if (fp && fp[0] == '0') return false;
+    const char* gen = getenv("SVNET_EDGE_GENERIC");    // the generic kernel reads the P | Q table, not the float4 one
+    if (gen && gen[0] == '1') return false;
     if (k != 20) return false;
     for (const ftc_shape& s : kFShapes)
         if (s.cs == cs && s.cv == cv && s.co == co && s.cvo == cvo) return true;

@@ -154,7 +154,8 @@ extern "C" int svnet_linear_rows_ws(const svnet_gemm_params* p, void* workspace,
         if (h < 0) return h;
         if (h == 1) return SVNET_OK;
     }
-    SV_REQUIRE(!p->c4, "svnet_linear_rows: the c4 table layout needs the tcgen05 vector-linear path (sign_w, G == 3, K <= 96, N <= 256)");
+    SV_REQUIRE(!p->c4, "svnet_linear_rows: the c4 table layout needs the tcgen05 vector-linear path (G == 3, K <= 96, N <= 256, "
+                       "no bias / BN / activation; full-precision weights also need SVNET_TCGEN05 and SVNET_VLINEAR_FP_TC not 0)");
     {   // binary-weight vector linears: exact-split bf16 mma.sync kernel (gemm_tc.cu)
         const int h = svnet_signlinear_tc_dispatch(p, st);
         if (h < 0) return h;

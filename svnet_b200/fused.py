@@ -50,6 +50,12 @@ def native_forward(model, kind, x, extra=None):
     if x.device.index != torch.cuda.current_device():
         with torch.cuda.device(x.device):
             return native_forward(model, kind, x, extra)
+    # the C entry runs edge layers 2..4 on the tensor-core kernels only; where a switch (SVNET_EDGE_TC=0,
+    # SVNET_VLINEAR_FP_TC=0, ...) takes them off, the module path below picks the kernel
+    covered = nv.edge_tc_weight_bytes if binary else nv.edge_fp_tc_weight_bytes
+    for blk in (model.conv2, model.conv3, model.conv4):
+        if covered(blk.in_dims[0] // 2, blk.in_dims[1] // 2, blk.out_dims[0], blk.out_dims[1], k) == 0:
+            return None
     from .native_model import NativeModel
     names = [n for n, t in model.state_dict().items() if t.dtype == torch.float32] if "_sv_native_names" not in model.__dict__ \
         else model.__dict__["_sv_native_names"]
