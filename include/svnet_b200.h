@@ -219,7 +219,8 @@ int svnet_edge_tc_pack_w(const float* W1, int ldw, int Cs, int Cv, int Cout, uns
 /* The same for the full-precision edge layers (sv_layers.py:29-31,186-190; csrc/edge_fp_tc.cu): the q part of linear1
  * (K = 6 Cv) runs on tcgen05 as six products of exact three-way bf16 splits (fp32-grade), the s part comes from the
  * per-point table `Yab` in the epilogue.  svnet_edge_fp_tc_weight_bytes() is 0 for shapes / k the kernel does not cover
- * (covered: the three fp edge-layer shapes of SV_DGCNN_CLS at k = 20; SVNET_EDGE_FP_TC=0 disables the path);
+ * (covered: the three fp edge-layer shapes of SV_DGCNN_CLS at k = 20 and those of SV_DGCNN_PSEG at k = 20 and 40 -- a set of
+ * (shape, k) pairs: the classifier's shapes at k = 40 are not covered; SVNET_EDGE_FP_TC=0 disables the path);
  * svnet_edge_fp_tc_pack_w() turns conv.linear1.weight [Cout][2Cs + 6Cv] into the three weight planes.  A full-precision
  * svnet_svblock_edge_fwd call takes this kernel when `W1tc` (those planes), `tab4` (float4 table, full-precision weights)
  * and `Yab` are set; `W1q_t` and `PQ` may then be NULL. */
@@ -356,6 +357,32 @@ typedef struct {
 size_t svnet_seg_head_workspace_bytes(const svnet_seg_head_params* p);
 int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspace, size_t workspace_bytes, void* stream);
 
+/* The same head of the full-precision model (binary = False: plain Conv1d weights, no beta / scale) as one call.  conv8's
+ * input is [glob[b] repeated over the points | svfuse1(s_cat, v_cat)]; its per-cloud part W8[:, :Kc] glob[b] is computed
+ * once per cloud and added to every point's W8[:, Kc:] u before BN + LeakyReLU, so the (B*N, Kc + Cs + 3Cv) table is never
+ * written.  Every linear (per-cloud term, conv8 .. conv11) goes through svnet_linear_rows_ws as the layer-by-layer calls do:
+ * the three-plane tcgen05 fp linear where it covers (K, N), e.g. not conv11 with fewer than 32 parts (chosen by (K, N) only:
+ * a cloud's logits do not depend on its batch); tolerance-level against the layer-by-layer calls (conv8's K is split).
+ * svnet_seg_head_fp_workspace_bytes() is 0 when the per-point conv8 (K = Cs + 3Cv, C8), which carries the per-cloud term,
+ * is not covered by the tcgen05 linear (SVNET_LINEAR_TC=0).
+ *   sv / Wz1      svfuse1's input and its v2s weight [3][Cv] (full precision: no scale); its (B*N, Cs + 3Cv) rows go to
+ *                 the workspace
+ *   glob [B][ldg] the Kc per-cloud-constant leading input channels of conv8
+ *   W8 [C8][Kc + Cs + 3Cv], W9 [C9][C8], W10 [C10][C9] with folded BatchNorm affines; W11 [parts][C10] */
+typedef struct {
+    svnet_view sv;
+    int B; long N;
+    const float* Wz1;
+    const float* glob; int ldg; int Kc;
+    const float* W8; const float* bn8_a; const float* bn8_c; int C8;
+    const float* W9; const float* bn9_a; const float* bn9_c; int C9;
+    const float* W10; const float* bn10_a; const float* bn10_c; int C10;
+    const float* W11; int parts;
+    float* logits;        /* [B][parts][N] */
+} svnet_seg_head_fp_params;
+size_t svnet_seg_head_fp_workspace_bytes(const svnet_seg_head_fp_params* p);
+int svnet_seg_head_fp_fwd(const svnet_seg_head_fp_params* p, void* workspace, size_t workspace_bytes, void* stream);
+
 /* VectorBN on materialised rows (module-level parity for sv_layers.VectorBN, :86-102):
  * v [rows][3][C] contiguous -> out. */
 int svnet_vector_bn_rows(const float* v, long rows, int C, const float* bn_a, const float* bn_c, float* out,
@@ -382,7 +409,7 @@ int svnet_svfuse_pool(const svnet_view* in, int B, long rows_per_cloud, const fl
  * without the 'module.' prefix (SURVEY 8(a) a-keys), fp32, contiguous -- copies what it needs and packs it once (sign
  * bit-planes, folded BatchNorm affines, tensor-core operand bytes, per-point table weights); it synchronises `stream` before
  * it returns, the caller's tensors may then be freed.  Covered: kind "SV_DGCNN_CLS", k = 20 (binary = 1 also k = 40); kind
- * "SV_DGCNN_PSEG" below.
+ * "SV_DGCNN_PSEG" below.  A state_dict that lacks a tensor of the kind / precision asked for fails with its name.
  * svnet_model_forward(): x [B][3][N] -> logits [B][num_class] on `stream`, with svnet_model_workspace_bytes(m, B, N) bytes of
  * caller-owned scratch (256-byte aligned; 0: shape not covered -- 64 <= N <= 4096).  It allocates
  * nothing and never synchronises the host, so it can be captured into a CUDA graph; inside, the work forks from `stream` onto
@@ -397,8 +424,10 @@ size_t svnet_model_workspace_bytes(const svnet_model* m, int B, int N);
 int svnet_model_forward(const svnet_model* m, const float* x, int B, int N, float* logits, void* workspace,
                         size_t workspace_bytes, void* stream);
 void svnet_model_destroy(svnet_model* m);
-/* kind "SV_DGCNN_PSEG" (models/sv_dgcnn_partseg.py:40-128; binary = 1, k = 20 or 40, num_class = number of parts):
- * x [B][3][N], label_onehot [B][16] -> logits [B][parts][N], with svnet_model_seg_workspace_bytes() bytes of scratch. */
+/* kind "SV_DGCNN_PSEG" (models/sv_dgcnn_partseg.py:40-128; binary = 1 or 0, k = 20 or 40, num_class = number of parts):
+ * x [B][3][N], label_onehot [B][16] -> logits [B][parts][N], with svnet_model_seg_workspace_bytes() bytes of scratch.
+ * Full precision (binary = 0): the state_dict has no beta / scale tensors; conv5 / conv6 are dense linears over
+ * u = [s | v2s(v)], svfuse1..3 plain v2s, and the head is svnet_seg_head_fp_fwd -- the same calls as the nn.Module path. */
 size_t svnet_model_seg_workspace_bytes(const svnet_model* m, int B, int N);
 int svnet_model_forward_seg(const svnet_model* m, const float* x, const float* label_onehot, int B, int N, float* logits,
                             void* workspace, size_t workspace_bytes, void* stream);

@@ -28,7 +28,7 @@ EXPORTS = [
     "svnet_edge_tc_weight_bytes", "svnet_edge_tc_table_cols", "svnet_edge_tc_pack_w", "svnet_allgather_logits",
     "svnet_edge_fp_tc_weight_bytes", "svnet_edge_fp_tc_pack_w", "svnet_seg_head_fwd", "svnet_seg_head_workspace_bytes",
     "svnet_model_create", "svnet_model_workspace_bytes", "svnet_model_forward", "svnet_model_destroy",
-    "svnet_model_seg_workspace_bytes", "svnet_model_forward_seg",
+    "svnet_model_seg_workspace_bytes", "svnet_model_forward_seg", "svnet_seg_head_fp_workspace_bytes", "svnet_seg_head_fp_fwd",
 ]
 
 
@@ -70,6 +70,14 @@ class SegHeadParams(ctypes.Structure):
                 ("C10", c_int), ("W11", c_void_p), ("parts", c_int), ("logits", c_void_p)]
 
 
+class SegHeadFpParams(ctypes.Structure):
+    _fields_ = [("sv", View), ("B", c_int), ("N", c_long), ("Wz1", c_void_p), ("glob", c_void_p), ("ldg", c_int), ("Kc", c_int),
+                ("W8", c_void_p), ("bn8_a", c_void_p), ("bn8_c", c_void_p), ("C8", c_int),
+                ("W9", c_void_p), ("bn9_a", c_void_p), ("bn9_c", c_void_p), ("C9", c_int),
+                ("W10", c_void_p), ("bn10_a", c_void_p), ("bn10_c", c_void_p), ("C10", c_int),
+                ("W11", c_void_p), ("parts", c_int), ("logits", c_void_p)]
+
+
 class TensorRef(ctypes.Structure):           # svnet_tensor
     _fields_ = [("name", ctypes.c_char_p), ("data", c_void_p), ("numel", c_long)]
 
@@ -102,6 +110,7 @@ def lib():
         l.svnet_edge_tc_weight_bytes.restype = ctypes.c_size_t
         l.svnet_edge_fp_tc_weight_bytes.restype = ctypes.c_size_t
         l.svnet_seg_head_workspace_bytes.restype = ctypes.c_size_t
+        l.svnet_seg_head_fp_workspace_bytes.restype = ctypes.c_size_t
         l.svnet_model_workspace_bytes.restype = ctypes.c_size_t
         l.svnet_model_workspace_bytes.argtypes = [c_void_p, c_int, c_int]
         l.svnet_model_seg_workspace_bytes.restype = ctypes.c_size_t
@@ -327,6 +336,33 @@ def seg_head_fwd(view, B, N, Wz1, zscale1, glob, layers, W11, sv_bits=None):
     return out
 
 
+def seg_head_fp_fwd(view, B, N, Wz1, glob, layers, W11):
+    """svnet_seg_head_fp_fwd: conv8 -> conv9 -> conv10 -> conv11 of the full-precision SV_DGCNN_PSEG in one call.  ``view`` =
+    (s_cat, v_cat), svfuse1's input; ``layers`` = three (W (Cout, K) contiguous, (bn_a, bn_c)) for conv8 / conv9 / conv10, conv8's
+    W over [glob | svfuse1 rows].  Returns (B, parts, N), or None when the per-point conv8 is not covered by the tensor-core linear."""
+    glob, W11 = _dev(glob), _dev(W11)
+    p = SegHeadFpParams()
+    p.sv, p.B, p.N, p.Wz1 = view, B, N, _dev(Wz1).data_ptr()
+    p.glob, p.ldg, p.Kc = glob.data_ptr(), glob.stride(0), glob.shape[1]
+    (W8, bn8), (W9, bn9), (W10, bn10) = layers
+    p.W8, p.bn8_a, p.bn8_c, p.C8 = _dev(W8).data_ptr(), bn8[0].data_ptr(), bn8[1].data_ptr(), W8.shape[0]
+    p.W9, p.bn9_a, p.bn9_c, p.C9 = _dev(W9).data_ptr(), bn9[0].data_ptr(), bn9[1].data_ptr(), W9.shape[0]
+    p.W10, p.bn10_a, p.bn10_c, p.C10 = _dev(W10).data_ptr(), bn10[0].data_ptr(), bn10[1].data_ptr(), W10.shape[0]
+    p.W11, p.parts = W11.data_ptr(), W11.shape[0]
+    nbytes = int(lib().svnet_seg_head_fp_workspace_bytes(ctypes.byref(p)))
+    if nbytes == 0:
+        return None
+    out = torch.empty((B, W11.shape[0], N), dtype=torch.float32, device=glob.device)
+    p.logits = out.data_ptr()
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=glob.device)
+    _call("svnet_seg_head_fp_fwd", ctypes.byref(p), _ptr(ws), ctypes.c_size_t(nbytes), _stream())
+    # kernels behind the one call: svfuse1's rows, per linear pack + tensor-core GEMM (or one CUDA-core kernel), transpose
+    Kp = view.Cs + 3 * view.Cv
+    shapes = [(p.Kc, p.C8), (Kp, p.C8), (p.C8, p.C9), (p.C9, p.C10), (p.C10, p.parts)]
+    LAUNCHES[0] += 1 + sum(2 if linear_tc_bytes(K, N) else 1 for K, N in shapes)
+    return out
+
+
 def model_create(kind, k, binary, num_class, state_dict):
     """svnet_model_create from a state_dict of CUDA fp32 tensors ('module.' prefixes are stripped); returns the handle."""
     items = [(n[7:] if n.startswith("module.") else n, t) for n, t in state_dict.items() if t.dtype == torch.float32]
@@ -443,6 +479,13 @@ def linear_rows(A, lda_g, lda_x, G, M, K, W, N, C, ldc_g, ldc_x, sign_w=False, c
     _call("svnet_linear_rows_ws", ctypes.byref(p), _ptr(ws), ctypes.c_size_t(nbytes), _stream())
     if nbytes > 0:
         LAUNCHES[0] += 1
+
+
+def linear_tc_bytes(K, N):
+    """Scratch of the three-plane tensor-core fp linear for a plain (K -> N) layer; 0 when it does not cover the shape."""
+    p = GemmParams()
+    p.G, p.M, p.K, p.N, p.ldw = 1, 1, K, N, K
+    return int(lib().svnet_linear_workspace_bytes(ctypes.byref(p)))
 
 
 def vector_bn_rows(v, bn_a, bn_c):

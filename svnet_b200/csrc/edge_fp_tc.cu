@@ -429,8 +429,13 @@ int launch_ftc(const svnet_edge_params* p, cudaStream_t st)
     return SVNET_OK;
 }
 
-struct ftc_shape { int cs, cv, co, cvo; };
-const ftc_shape kFShapes[] = {{32, 10, 32, 10}, {32, 10, 64, 21}, {64, 21, 128, 42}};
+// The instantiated (shape, k) pairs: the three fp edge layers of SV_DGCNN_CLS at k = 20 and of SV_DGCNN_PSEG at k = 20 / 40.
+// svnet_edge_fp_tc_weight_bytes goes through ftc_covered, which reads this list; svnet_edge_fp_tc_dispatch has one FCASE per
+// entry and no other, so a covered layer always finds its kernel.
+struct ftc_case { int cs, cv, co, cvo, k; };
+const ftc_case kFCases[] = {{32, 10, 32, 10, 20}, {32, 10, 64, 21, 20}, {64, 21, 128, 42, 20},
+                            {32, 16, 32, 16, 20}, {32, 16, 64, 24, 20}, {64, 24, 128, 40, 20},
+                            {32, 16, 32, 16, 40}, {32, 16, 64, 24, 40}, {64, 24, 128, 40, 40}};
 
 bool ftc_covered(int cs, int cv, int co, int cvo, int k)
 {
@@ -442,9 +447,8 @@ bool ftc_covered(int cs, int cv, int co, int cvo, int k)
     if (fp && fp[0] == '0') return false;
     const char* gen = getenv("SVNET_EDGE_GENERIC");    // the generic kernel reads the P | Q table, not the float4 one
     if (gen && gen[0] == '1') return false;
-    if (k != 20) return false;
-    for (const ftc_shape& s : kFShapes)
-        if (s.cs == cs && s.cv == cv && s.co == co && s.cvo == cvo) return true;
+    for (const ftc_case& s : kFCases)
+        if (s.cs == cs && s.cv == cv && s.co == co && s.cvo == cvo && s.k == k) return true;
     return false;
 }
 
@@ -483,6 +487,12 @@ int svnet_edge_fp_tc_dispatch(const svnet_edge_params* p, cudaStream_t st)
     FCASE(32, 10, 32, 10, 20)
     FCASE(32, 10, 64, 21, 20)
     FCASE(64, 21, 128, 42, 20)
+    FCASE(32, 16, 32, 16, 20)
+    FCASE(32, 16, 64, 24, 20)
+    FCASE(64, 24, 128, 40, 20)
+    FCASE(32, 16, 32, 16, 40)
+    FCASE(32, 16, 64, 24, 40)
+    FCASE(64, 24, 128, 40, 40)
 #undef FCASE
     return 0;
 }

@@ -157,6 +157,8 @@ struct tc3_args {
     int act;
     float* C;
     long ldc;
+    const float* rowadd;     // optional: + rowadd[(row / rows_per_add) * ld_add + channel] before BN (a per-cloud term)
+    long rows_per_add, ld_add;
 };
 
 __global__ void __launch_bounds__(NTH, 1) gemm_tc3_kernel(tc3_args p)
@@ -298,10 +300,22 @@ __global__ void __launch_bounds__(NTH, 1) gemm_tc3_kernel(tc3_args p)
                 if (!cok) continue;
                 float* op = p.C + rb * p.ldc + c;
                 const int nrow = (int)min(32L, p.rows - rb);
+                // row group of the first row and the first row of the next group: one division per 32 rows
+                const float* addp = nullptr;
+                long next_group = 0;
+                if (p.rowadd) {
+                    const long g = rb / p.rows_per_add;
+                    addp = p.rowadd + g * p.ld_add + c;
+                    next_group = (g + 1) * p.rows_per_add;
+                }
 #pragma unroll
                 for (int j = 0; j < 32; ++j) {
                     if (j < nrow) {
                         float v = d[j] * cs + bi;            // (colscale == 1 / bias == 0 when absent)
+                        if (addp) {
+                            while (rb + j >= next_group) { addp += p.ld_add; next_group += p.rows_per_add; }
+                            v += __ldg(addp);
+                        }
                         v = v * a1 + c1;
                         op[(long)j * p.ldc] = sv_act(v, p.act);
                     }
@@ -339,8 +353,10 @@ size_t svnet_linear_tc3_workspace(const svnet_gemm_params* p)
     return wb;
 }
 
-// Returns 1 if handled, 0 if the caller should use the CUDA-core kernel, < 0 on error.
-int svnet_linear_tc3_dispatch(const svnet_gemm_params* p, void* workspace, size_t workspace_bytes, cudaStream_t st)
+// svnet_linear_tc3_dispatch with a per-row-group addend (library-internal: the full-precision part-segmentation head adds conv8's per-cloud
+// term, rowadd [rows / rows_per_add][ld_add], to every point of the cloud before BN).
+int svnet_linear_tc3_rowadd(const svnet_gemm_params* p, const float* rowadd, long rows_per_add, long ld_add, void* workspace,
+                            size_t workspace_bytes, cudaStream_t st)
 {
     int MT, NKC;
     size_t wb, smem;
@@ -358,8 +374,15 @@ int svnet_linear_tc3_dispatch(const svnet_gemm_params* p, void* workspace, size_
     a.Wtc = static_cast<const unsigned char*>(workspace);
     a.colscale = p->colscale; a.bias = p->bias; a.bn_a = p->bn_a; a.bn_c = p->bn_c; a.act = p->act;
     a.C = p->C; a.ldc = p->ldc_g;
+    a.rowadd = rowadd; a.rows_per_add = rows_per_add; a.ld_add = ld_add;
     SV_CUDA(cudaFuncSetAttribute(gemm_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     gemm_tc3_kernel<<<dim3(row_tiles, sv_cdiv(MT, mt_per_cta)), NTH, smem, st>>>(a);
     SV_CHECK_LAUNCH("svnet_linear_rows(tcgen05 x3)");
     return 1;
+}
+
+// Returns 1 if handled, 0 if the caller should use the CUDA-core kernel, < 0 on error.
+int svnet_linear_tc3_dispatch(const svnet_gemm_params* p, void* workspace, size_t workspace_bytes, cudaStream_t st)
+{
+    return svnet_linear_tc3_rowadd(p, nullptr, 1, 0, workspace, workspace_bytes, st);
 }

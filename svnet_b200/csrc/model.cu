@@ -17,6 +17,8 @@
 // Covered: k = 20 (binary also 40: the shapes of the tensor-core edge kernels), 64 <= N <= 4096.  The list of calls above is
 // the binary model's; the full-precision model takes svnet_linear_rows_ws where the binary one takes the sign-word kernels
 // (sv_dgcnn_cls.py in this package shows both).
+// The part-segmentation model (svnet_model_forward_seg, binary or full precision, k = 20 or 40) follows below; its
+// full-precision head is svnet_seg_head_fp_fwd (conv8's per-cloud part once per cloud).
 #include "common.cuh"
 #include <stdlib.h>
 #include <string.h>
@@ -44,7 +46,7 @@ struct svnet_model {
     float *h1_W, *h2_W;              // full-precision head
     // part segmentation: svfuse1 / 2 / 3, conv7 (labels), conv8 .. conv11
     float *f1_Wz, *f1_zs, *f2_Wz, *f2_zs, *f3_Wz, *f3_zs, *c7_W, *c7_a, *c7_c;
-    struct SegConv { float *beta, *scale, *bn_a, *bn_c; uint32_t *bits, *bits_c; int Cin, Cout; } c8, c9, c10;
+    struct SegConv { float *beta, *scale, *bn_a, *bn_c; uint32_t *bits, *bits_c; float* W; int Cin, Cout; } c8, c9, c10;   // W: fp
     float* c11_W;
     int C6s, C6v, Kc;
     // launch structure of svnet_model_forward: two sub-batch streams, each with an auxiliary stream for the chains that do
@@ -179,6 +181,28 @@ size_t plan_trunk(const svnet_model* m, int B, int N, fwd_plan* pl)
     return o;
 }
 
+// the largest scratch of the plain fp linear (rows x K -> Nc) and `lb`
+size_t max_lin(size_t lb, long rows, int K, int Nc)
+{
+    svnet_gemm_params q = {};
+    q.G = 1; q.M = rows; q.N = Nc; q.K = K;
+    const size_t b = svnet_linear_workspace_bytes(&q);
+    return b > lb ? b : lb;
+}
+
+// full precision, classifier and part segmentation: the Ya | Yb table of the edge layers, conv5's u = [s | v2s(v)] rows and its
+// scalar output; returns the running offset, *lb = the largest scratch of those linears (Ya | Yb and conv5, one at a time)
+size_t plan_fp_rows(const svnet_model* m, long R, int K5, fwd_plan* pl, size_t o, size_t* lb)
+{
+    pl->yab = o; o += up256(sizeof(float) * R * 2 * m->conv[3].Cout);
+    pl->u5 = o; o += up256(sizeof(float) * R * K5);
+    pl->s5 = o; o += up256(sizeof(float) * R * m->C5s);
+    size_t b = max_lin(0, R, K5, m->C5s);
+    for (int l = 1; l < 4; ++l) b = max_lin(b, R, m->conv[l].Cs, 2 * m->conv[l].Cout);
+    *lb = b;
+    return o;
+}
+
 bool make_fwd_plan(const svnet_model* m, int B, int N, fwd_plan* pl)
 {
     const long R = (long)B * N;
@@ -195,25 +219,10 @@ bool make_fwd_plan(const svnet_model* m, int B, int N, fwd_plan* pl)
         // full precision: Ya | Yb table of the edge layers, conv5's u = [s | v2s(v)] rows and scalar output, head layer 1
         pl->bits = pl->mask = pl->nvalid = pl->blp = 0;
         pl->blp_bytes = pl->bl_bytes = 0;
-        pl->yab = o; o += up256(sizeof(float) * R * 2 * m->conv[3].Cout);
-        pl->u5 = o; o += up256(sizeof(float) * R * K5);
-        pl->s5 = o; o += up256(sizeof(float) * R * m->C5s);
+        size_t lb;
+        o = plan_fp_rows(m, R, K5, pl, o, &lb);
         pl->h1 = o; o += up256(sizeof(float) * B * m->h1);
-        svnet_gemm_params q = {};
-        q.G = 1; q.M = R; q.N = m->C5s; q.K = K5; q.bn_a = reinterpret_cast<const float*>(1); q.act = SVNET_ACT_LEAKY;
-        size_t lb = svnet_linear_workspace_bytes(&q);
-        for (int l = 1; l < 4; ++l) {
-            svnet_gemm_params y = {};
-            y.G = 1; y.M = R; y.N = 2 * m->conv[l].Cout; y.K = m->conv[l].Cs;
-            const size_t b2 = svnet_linear_workspace_bytes(&y);
-            lb = b2 > lb ? b2 : lb;
-        }
-        {
-            svnet_gemm_params y = {};
-            y.G = 1; y.M = B; y.N = m->h1; y.K = 2 * m->Cf; y.bn_a = reinterpret_cast<const float*>(1); y.act = SVNET_ACT_LEAKY;
-            const size_t b2 = svnet_linear_workspace_bytes(&y);
-            lb = b2 > lb ? b2 : lb;
-        }
+        lb = max_lin(lb, B, 2 * m->Cf, m->h1);
         pl->lin_bytes = lb;
         pl->lin = o; o += up256(lb);
         pl->fuse_bytes = svnet_svfuse_pool_workspace(B, m->C5v, N);
@@ -254,8 +263,8 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
     SV_REQUIRE(pseg || strcmp(kind, "SV_DGCNN_CLS") == 0,
                "svnet_model_create: kind '%s' not covered (SV_DGCNN_CLS, SV_DGCNN_PSEG; the PointNet models go through the nn.Module API)", kind);
     SV_REQUIRE(binary == 0 || binary == 1, "svnet_model_create: binary must be 0 or 1");
-    SV_REQUIRE(!pseg || binary, "svnet_model_create: the full-precision part-segmentation model goes through the nn.Module API");
-    SV_REQUIRE(k == 20 || (binary && k == 40), "svnet_model_create: k = %d not covered (the tensor-core edge kernels' shapes: 20, binary also 40)", k);
+    SV_REQUIRE(k == 20 || (k == 40 && (binary || pseg)),
+               "svnet_model_create: k = %d not covered (the tensor-core edge kernels' shapes: 20; binary and part segmentation also 40)", k);
     SV_REQUIRE(num_class >= 1, "svnet_model_create: bad num_class");
     svnet_model* m = new svnet_model();
     m->k = k; m->ncls = num_class; m->binary = binary; m->pseg = pseg ? 1 : 0;
@@ -356,12 +365,18 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
     if (L.ok && pseg) {
         m->C6s = cs_out[5]; m->C6v = cv_out[5];
         const int cs_cat = 256, cv_cat = 96;
-        m->f1_Wz = L.signed_copy("svfuse1.v2s.linear.weight", 3 * cv_cat);
-        m->f1_zs = L.dup("svfuse1.v2s.linear.scale", 3);
-        m->f2_Wz = L.signed_copy("svfuse2.v2s.linear.weight", 3 * m->C6v);
-        m->f2_zs = L.dup("svfuse2.v2s.linear.scale", 3);
-        m->f3_Wz = L.signed_copy("svfuse3.v2s.linear.weight", 3 * m->C5v);
-        m->f3_zs = L.dup("svfuse3.v2s.linear.scale", 3);
+        if (binary) {
+            m->f1_Wz = L.signed_copy("svfuse1.v2s.linear.weight", 3 * cv_cat);
+            m->f1_zs = L.dup("svfuse1.v2s.linear.scale", 3);
+            m->f2_Wz = L.signed_copy("svfuse2.v2s.linear.weight", 3 * m->C6v);
+            m->f2_zs = L.dup("svfuse2.v2s.linear.scale", 3);
+            m->f3_Wz = L.signed_copy("svfuse3.v2s.linear.weight", 3 * m->C5v);
+            m->f3_zs = L.dup("svfuse3.v2s.linear.scale", 3);
+        } else {      // full precision: plain v2s weights, no scales (zscale = NULL below)
+            m->f1_Wz = L.dup("svfuse1.v2s.linear.weight", 3 * cv_cat);
+            m->f2_Wz = L.dup("svfuse2.v2s.linear.weight", 3 * m->C6v);
+            m->f3_Wz = L.dup("svfuse3.v2s.linear.weight", 3 * m->C5v);
+        }
         m->c7_W = L.dup("conv7.0.weight", 64 * 16);
         L.fold("conv7.1", 64, &m->c7_a, &m->c7_c);
         // conv8 input = [glob (per cloud): s5 max | v2s(v5) max | svfuse2(conv6) | conv7(label)] ++ [svfuse1(s_cat, v_cat) per point]
@@ -370,11 +385,17 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
         auto seg_conv = [&](const char* name, int Cin, int Cout, svnet_model::SegConv* c, int split) {
             const std::string p = std::string(name) + ".";
             c->Cin = Cin; c->Cout = Cout;
+            c->beta = c->scale = c->W = nullptr;
+            c->bits = c->bits_c = nullptr;
+            if (!binary) {     // full precision: the weight [Cout][Cin] as it is and the folded BN
+                c->W = L.dup(p + "0.weight", (long)Cout * Cin);
+                L.fold(p + "1", Cout, &c->bn_a, &c->bn_c);
+                return;
+            }
             const svnet_tensor* w = L.find(p + "0.weight", (long)Cout * Cin);
             c->beta = L.dup(p + "0.beta", Cin);
             c->scale = L.dup(p + "0.scale", Cout);
             L.fold(p + "1", Cout, &c->bn_a, &c->bn_c);
-            c->bits = c->bits_c = nullptr;
             if (!w) return;
             if (split > 0) {
                 // sign planes of the per-cloud columns [:, :split] and of the per-point columns [:, split:]
@@ -726,6 +747,7 @@ namespace {
 struct seg_plan2 {
     fwd_plan t;
     size_t bits8, mask8, nvalid8, bits5, mask5, nvalid5, blp, s5, v5, glob, vp, v6, bits6, mask6, nvalid6, fuse, head, total;
+    size_t u6;            // full precision: conv6's rows u = [s | v2s(v)] (conv5's: t.u5)
     size_t blp_bytes, bl_bytes, fuse_bytes, head_bytes;
 };
 
@@ -741,10 +763,51 @@ svnet_seg_head_params seg_head_params(const svnet_model* m, int B, int N)
     return h;
 }
 
+svnet_seg_head_fp_params seg_head_fp_params(const svnet_model* m, int B, int N)
+{
+    svnet_seg_head_fp_params h = {};
+    h.sv.Cs = 256; h.sv.Cv = 96; h.sv.lds = 256; h.sv.ldv = 3 * 96; h.sv.xs = 96;
+    h.B = B; h.N = N; h.Wz1 = m->f1_Wz; h.ldg = m->Kc; h.Kc = m->Kc;
+    h.W8 = m->c8.W; h.bn8_a = m->c8.bn_a; h.bn8_c = m->c8.bn_c; h.C8 = m->c8.Cout;
+    h.W9 = m->c9.W; h.bn9_a = m->c9.bn_a; h.bn9_c = m->c9.bn_c; h.C9 = m->c9.Cout;
+    h.W10 = m->c10.W; h.bn10_a = m->c10.bn_a; h.bn10_c = m->c10.bn_c; h.C10 = m->c10.Cout;
+    h.W11 = m->c11_W; h.parts = m->ncls;
+    return h;
+}
+
+// full precision: trunk (+ Ya | Yb table), conv5's u rows and scalar output, the global branch, the fp head
+bool make_seg_plan_fp(const svnet_model* m, int B, int N, seg_plan2* pl, size_t o)
+{
+    const long R = (long)B * N;
+    const int Kp = pl->t.Cs_cat + 3 * pl->t.Cv_cat, K6 = m->C5s + 3 * m->C5v;
+    pl->bits8 = pl->mask8 = pl->nvalid8 = pl->bits5 = pl->mask5 = pl->nvalid5 = pl->blp = pl->s5 = pl->bits6 = pl->mask6 = pl->nvalid6 = 0;
+    pl->blp_bytes = pl->bl_bytes = 0;
+    size_t lb;
+    o = plan_fp_rows(m, R, Kp, &pl->t, o, &lb);
+    pl->v5 = o; o += up256(sizeof(float) * R * 3 * m->C5v);
+    pl->glob = o; o += up256(sizeof(float) * B * m->Kc);
+    pl->vp = o; o += up256(sizeof(float) * B * 3 * m->C5v);
+    pl->u6 = o; o += up256(sizeof(float) * B * K6);
+    pl->v6 = o; o += up256(sizeof(float) * B * 3 * m->C6v);
+    // scratch of the fp linears outside the head (one at a time): plan_fp_rows' and conv6's
+    lb = max_lin(lb, B, K6, m->C6s);
+    pl->t.lin_bytes = lb;
+    pl->t.lin = o; o += up256(lb);
+    pl->fuse_bytes = svnet_svfuse_pool_workspace(B, m->C5v, N);
+    pl->fuse = o; o += up256(pl->fuse_bytes);
+    const svnet_seg_head_fp_params h = seg_head_fp_params(m, B, N);
+    pl->head_bytes = svnet_seg_head_fp_workspace_bytes(&h);
+    pl->head = o; o += up256(pl->head_bytes);
+    pl->total = o;
+    return pl->t.knn_bytes > 0 && pl->head_bytes > 0;
+}
+
 bool make_seg_plan(const svnet_model* m, int B, int N, seg_plan2* pl)
 {
     const long R = (long)B * N;
     size_t o = plan_trunk(m, B, N, &pl->t);
+    if (!m->binary) return make_seg_plan_fp(m, B, N, pl, o);
+    pl->u6 = 0;
     const int cs = pl->t.Cs_cat, cv = pl->t.Cv_cat;
     const int Kp = cs + 3 * cv, Kpw = (Kp + 31) / 32;
     const int K6 = m->C5s + 3 * m->C5v, K6w = (K6 + 31) / 32;
@@ -822,8 +885,10 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
     uint32_t* bits8 = reinterpret_cast<uint32_t*>(ws + pl.bits8);
     uint32_t* mask8 = reinterpret_cast<uint32_t*>(ws + pl.mask8);
     int32_t* nvalid8 = reinterpret_cast<int32_t*>(ws + pl.nvalid8);
-    rc = svnet_rows_prep(&cat, R, m->f1_Wz, m->f1_zs, nullptr, m->c8.beta + Kc, nullptr, 0, nullptr, bits8, mask8, nvalid8, sst);
-    if (rc != SVNET_OK) return rc;
+    if (m->binary) {
+        rc = svnet_rows_prep(&cat, R, m->f1_Wz, m->f1_zs, nullptr, m->c8.beta + Kc, nullptr, 0, nullptr, bits8, mask8, nvalid8, sst);
+        if (rc != SVNET_OK) return rc;
+    }
     // conv5 per point: scalar output only pooled (max) -> glob[:, :C5s]; vector output v5
     const svnet_model::Block& c5 = m->conv[4];
     float* glob = reinterpret_cast<float*>(ws + pl.glob);
@@ -831,19 +896,34 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
     uint32_t* bits5 = reinterpret_cast<uint32_t*>(ws + pl.bits5);
     uint32_t* mask5 = reinterpret_cast<uint32_t*>(ws + pl.mask5);
     int32_t* nvalid5 = reinterpret_cast<int32_t*>(ws + pl.nvalid5);
-    rc = svnet_rows_prep(&cat, R, c5.Wz, c5.zscale, nullptr, c5.beta, nullptr, 0, nullptr, bits5, mask5, nvalid5, sst);
-    if (rc != SVNET_OK) return rc;
-    if (pl.blp_bytes) {
-        rc = svnet_binlinear_pool_ws(bits5, mask5, R, Kp, c5.W1b, C5s, c5.scale1, c5.bn1_a, c5.bn1_c, N, glob, nullptr, Kc, ws + pl.blp,
-                                     pl.blp_bytes, sst);
+    if (!m->binary) {
+        // full precision: u = [s | v2s(v)] rows -> dense linear1 + BN + LeakyReLU -> max over the points (as the fp classifier)
+        float* u5 = reinterpret_cast<float*>(ws + pl.t.u5);
+        float* s5 = reinterpret_cast<float*>(ws + pl.t.s5);
+        rc = svnet_rows_prep(&cat, R, c5.Wz, nullptr, nullptr, nullptr, u5, Kp, nullptr, nullptr, nullptr, nullptr, sst);
         if (rc != SVNET_OK) return rc;
-    } else {
-        float* s5 = reinterpret_cast<float*>(ws + pl.s5);
-        rc = svnet_binlinear_rows_ws(bits5, mask5, nvalid5, R, Kp, c5.W1b, C5s, c5.scale1, nullptr, c5.bn1_a, c5.bn1_c, SVNET_ACT_LEAKY, nullptr,
-                                     1, s5, C5s, nullptr, pl.bl_bytes ? ws + pl.blp : nullptr, pl.bl_bytes, sst);
+        svnet_gemm_params q = {};
+        q.A = u5; q.lda_g = Kp; q.lda_x = 0; q.G = 1; q.W = c5.W1; q.ldw = Kp; q.M = R; q.N = C5s; q.K = Kp;
+        q.bn_a = c5.bn1_a; q.bn_c = c5.bn1_c; q.act = SVNET_ACT_LEAKY; q.C = s5; q.ldc_g = C5s; q.ldc_x = 0; q.groups_per_cloud = 1;
+        rc = svnet_linear_rows_ws(&q, ws + pl.t.lin, pl.t.lin_bytes, sst);
         if (rc != SVNET_OK) return rc;
         rc = svnet_pool_rows(s5, C5s, C5s, B, N, glob, nullptr, Kc, sst);
         if (rc != SVNET_OK) return rc;
+    } else {
+        rc = svnet_rows_prep(&cat, R, c5.Wz, c5.zscale, nullptr, c5.beta, nullptr, 0, nullptr, bits5, mask5, nvalid5, sst);
+        if (rc != SVNET_OK) return rc;
+        if (pl.blp_bytes) {
+            rc = svnet_binlinear_pool_ws(bits5, mask5, R, Kp, c5.W1b, C5s, c5.scale1, c5.bn1_a, c5.bn1_c, N, glob, nullptr, Kc, ws + pl.blp,
+                                         pl.blp_bytes, sst);
+            if (rc != SVNET_OK) return rc;
+        } else {
+            float* s5 = reinterpret_cast<float*>(ws + pl.s5);
+            rc = svnet_binlinear_rows_ws(bits5, mask5, nvalid5, R, Kp, c5.W1b, C5s, c5.scale1, nullptr, c5.bn1_a, c5.bn1_c, SVNET_ACT_LEAKY,
+                                         nullptr, 1, s5, C5s, nullptr, pl.bl_bytes ? ws + pl.blp : nullptr, pl.bl_bytes, sst);
+            if (rc != SVNET_OK) return rc;
+            rc = svnet_pool_rows(s5, C5s, C5s, B, N, glob, nullptr, Kc, sst);
+            if (rc != SVNET_OK) return rc;
+        }
     }
     if (aux) SV_CUDA(cudaEventRecord(eJ, aux));
     rc = svnet_gate_rows(s_cat, lds, lds, B, N, c5.G1, c5.G2, c5.H, c5.Cvo, gate, stream);
@@ -851,7 +931,8 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
     {
         svnet_gemm_params q = {};
         q.A = v_cat; q.lda_g = ldv; q.lda_x = xs; q.G = 3; q.W = c5.W2; q.ldw = c5.Cv; q.M = 3 * R; q.N = C5v; q.K = c5.Cv;
-        q.sign_w = 1; q.colscale = c5.scale2; q.bn_a = c5.bn2_a; q.bn_c = c5.bn2_c; q.vbn = 1; q.gate = gate; q.groups_per_cloud = N;
+        q.sign_w = m->binary; q.colscale = m->binary ? c5.scale2 : nullptr; q.bn_a = c5.bn2_a; q.bn_c = c5.bn2_c; q.vbn = 1; q.gate = gate;
+        q.groups_per_cloud = N;
         q.C = v5; q.ldc_g = 3 * C5v; q.ldc_x = C5v;
         rc = svnet_linear_rows_ws(&q, nullptr, 0, stream);
         if (rc != SVNET_OK) return rc;
@@ -874,17 +955,29 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
     uint32_t* bits6 = reinterpret_cast<uint32_t*>(ws + pl.bits6);
     uint32_t* mask6 = reinterpret_cast<uint32_t*>(ws + pl.mask6);
     int32_t* nvalid6 = reinterpret_cast<int32_t*>(ws + pl.nvalid6);
-    rc = svnet_rows_prep(&pv, B, c6.Wz, c6.zscale, nullptr, c6.beta, nullptr, 0, nullptr, bits6, mask6, nvalid6, stream);
-    if (rc != SVNET_OK) return rc;
-    rc = svnet_binlinear_rows_ws(bits6, mask6, nvalid6, B, C5s + 3 * C5v, c6.W1b, C6s, c6.scale1, nullptr, c6.bn1_a, c6.bn1_c, SVNET_ACT_LEAKY,
-                                 nullptr, 1, glob + C3, Kc, nullptr, nullptr, 0, stream);
-    if (rc != SVNET_OK) return rc;
+    if (m->binary) {
+        rc = svnet_rows_prep(&pv, B, c6.Wz, c6.zscale, nullptr, c6.beta, nullptr, 0, nullptr, bits6, mask6, nvalid6, stream);
+        if (rc != SVNET_OK) return rc;
+        rc = svnet_binlinear_rows_ws(bits6, mask6, nvalid6, B, C3, c6.W1b, C6s, c6.scale1, nullptr, c6.bn1_a, c6.bn1_c, SVNET_ACT_LEAKY,
+                                     nullptr, 1, glob + C3, Kc, nullptr, nullptr, 0, stream);
+        if (rc != SVNET_OK) return rc;
+    } else {
+        float* u6 = reinterpret_cast<float*>(ws + pl.u6);
+        rc = svnet_rows_prep(&pv, B, c6.Wz, nullptr, nullptr, nullptr, u6, C3, nullptr, nullptr, nullptr, nullptr, stream);
+        if (rc != SVNET_OK) return rc;
+        svnet_gemm_params q = {};
+        q.A = u6; q.lda_g = C3; q.lda_x = 0; q.G = 1; q.W = c6.W1; q.ldw = C3; q.M = B; q.N = C6s; q.K = C3;
+        q.bn_a = c6.bn1_a; q.bn_c = c6.bn1_c; q.act = SVNET_ACT_LEAKY; q.C = glob + C3; q.ldc_g = Kc; q.ldc_x = 0; q.groups_per_cloud = 1;
+        rc = svnet_linear_rows_ws(&q, ws + pl.t.lin, pl.t.lin_bytes, stream);
+        if (rc != SVNET_OK) return rc;
+    }
     rc = svnet_gate_rows(glob, Kc, C5s, B, 1, c6.G1, c6.G2, c6.H, c6.Cvo, gate, stream);
     if (rc != SVNET_OK) return rc;
     {
         svnet_gemm_params q = {};
         q.A = vp; q.lda_g = 3 * C5v; q.lda_x = C5v; q.G = 3; q.W = c6.W2; q.ldw = C5v; q.M = 3L * B; q.N = C6v; q.K = C5v;
-        q.sign_w = 1; q.colscale = c6.scale2; q.bn_a = c6.bn2_a; q.bn_c = c6.bn2_c; q.vbn = 1; q.gate = gate; q.groups_per_cloud = 1;
+        q.sign_w = m->binary; q.colscale = m->binary ? c6.scale2 : nullptr; q.bn_a = c6.bn2_a; q.bn_c = c6.bn2_c; q.vbn = 1; q.gate = gate;
+        q.groups_per_cloud = 1;
         q.C = v6; q.ldc_g = 3 * C6v; q.ldc_x = C6v;
         rc = svnet_linear_rows_ws(&q, nullptr, 0, stream);
         if (rc != SVNET_OK) return rc;
@@ -911,6 +1004,11 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
         SV_CUDA(cudaStreamWaitEvent(st, eJ, 0));
     }
     // segmentation head
+    if (!m->binary) {
+        svnet_seg_head_fp_params h = seg_head_fp_params(m, B, N);
+        h.sv = cat; h.glob = glob; h.logits = logits;
+        return svnet_seg_head_fp_fwd(&h, ws + pl.head, pl.head_bytes, stream);
+    }
     svnet_seg_head_params h = seg_head_params(m, B, N);
     h.glob = glob; h.bits8 = bits8; h.mask8 = mask8; h.nvalid8 = nvalid8; h.logits = logits;
     return svnet_seg_head_fwd(&h, ws + pl.head, pl.head_bytes, stream);

@@ -12,7 +12,16 @@
 //   * conv11: three-plane tcgen05 GEMM (csrc/gemm_tc3.cu) into a row-major scratch, then one tiled transpose.
 // Bit-identical to the same layers called one by one through svnet_rows_prep / svnet_binlinear_rows_ws /
 // svnet_linear_rows_ws (tests/test_gpu_parity.py::test_seg_head_call_equals_layerwise).
+//
+// svnet_seg_head_fp_fwd: the same head of the full-precision model.  svfuse1's rows u = [s | v2s(v)] go to the workspace;
+// conv8's per-cloud part W8[:, :Kc] glob[b] is one linear over the B clouds, added per point in the epilogue of the per-point
+// linear (K = Cs + 3Cv instead of Kc + Cs + 3Cv); conv9 .. conv11 as the module's fp Conv1d layers.  Every linear goes through
+// svnet_linear_rows_ws: the three-plane tcgen05 kernel (csrc/gemm_tc3.cu) where it covers (K, N), the CUDA-core chain otherwise
+// (conv11 with fewer than 32 parts); the per-point conv8, which carries the per-cloud term, needs the tcgen05 kernel.
 #include "common.cuh"
+
+int svnet_linear_tc3_rowadd(const svnet_gemm_params* p, const float* rowadd, long rows_per_add, long ld_add, void* workspace,
+                            size_t workspace_bytes, cudaStream_t st);
 
 namespace {
 
@@ -165,5 +174,113 @@ extern "C" int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspac
     if (rc != SVNET_OK) return rc;
     seg_transpose_kernel<<<dim3(sv_cdiv(p->N, 32), sv_cdiv(p->parts, 32), p->B), 256, 0, sv_stream(stream)>>>(hB, p->parts, p->N, p->logits);
     SV_CHECK_LAUNCH("svnet_seg_head_fwd(transpose)");
+    return SVNET_OK;
+}
+
+// ---- full-precision head ----------------------------------------------------------------------------------------------
+namespace {
+
+struct seg_fp_plan {
+    size_t u, cterm, hA, hB, lws, total, lws_bytes;
+};
+
+svnet_gemm_params fp_linear(const float* A, long lda, long M, int K, const float* W, int ldw, int N, const float* bn_a,
+                            const float* bn_c, int act, float* C, long ldc)
+{
+    svnet_gemm_params g = {};
+    g.A = A; g.lda_g = lda; g.lda_x = 0; g.G = 1;
+    g.W = W; g.ldw = ldw; g.M = M; g.N = N; g.K = K;
+    g.bn_a = bn_a; g.bn_c = bn_c; g.act = act;
+    g.C = C; g.ldc_g = ldc; g.ldc_x = 0; g.groups_per_cloud = 1;
+    return g;
+}
+
+// the five linears of the head, in call order: per-cloud term, conv8 (per point), conv9, conv10, conv11
+void fp_linears(const svnet_seg_head_fp_params* p, const float* u, float* cterm, float* hA, float* hB, svnet_gemm_params g[5])
+{
+    const long R = (long)p->B * p->N;
+    const int Kp = p->sv.Cs + 3 * p->sv.Cv, K8 = p->Kc + Kp;
+    g[0] = fp_linear(p->glob, p->ldg, p->B, p->Kc, p->W8, K8, p->C8, nullptr, nullptr, SVNET_ACT_NONE, cterm, p->C8);
+    g[1] = fp_linear(u, Kp, R, Kp, p->W8 ? p->W8 + p->Kc : nullptr, K8, p->C8, p->bn8_a, p->bn8_c, SVNET_ACT_LEAKY, hA, p->C8);
+    g[2] = fp_linear(hA, p->C8, R, p->C8, p->W9, p->C8, p->C9, p->bn9_a, p->bn9_c, SVNET_ACT_LEAKY, hB, p->C9);
+    g[3] = fp_linear(hB, p->C9, R, p->C9, p->W10, p->C9, p->C10, p->bn10_a, p->bn10_c, SVNET_ACT_LEAKY, hA, p->C10);
+    g[4] = fp_linear(hA, p->C10, R, p->C10, p->W11, p->C10, p->parts, nullptr, nullptr, SVNET_ACT_NONE, hB, p->parts);
+}
+
+// false: the per-point conv8 (the only linear with the per-cloud addend) is not covered by the tensor-core linear
+bool make_fp_plan(const svnet_seg_head_fp_params* p, seg_fp_plan* pl)
+{
+    const long R = (long)p->B * p->N;
+    const int Kp = p->sv.Cs + 3 * p->sv.Cv;
+    const int hAc = p->C8 > p->C10 ? p->C8 : p->C10;
+    const int hBc = p->C9 > p->parts ? p->C9 : p->parts;
+    size_t o = 0;
+    pl->u = o; o += a256((size_t)R * Kp * 4);
+    pl->cterm = o; o += a256((size_t)p->B * p->C8 * 4);
+    pl->hA = o; o += a256((size_t)R * hAc * 4);
+    pl->hB = o; o += a256((size_t)R * hBc * 4);
+    svnet_gemm_params g[5];
+    fp_linears(p, nullptr, nullptr, nullptr, nullptr, g);
+    size_t lb = 0;
+    for (int i = 0; i < 5; ++i) {
+        const size_t b = svnet_linear_workspace_bytes(&g[i]);
+        lb = b > lb ? b : lb;
+    }
+    pl->lws_bytes = lb;
+    pl->lws = o; o += a256(lb);
+    pl->total = o;
+    return svnet_linear_workspace_bytes(&g[1]) > 0;
+}
+
+}  // namespace
+
+extern "C" size_t svnet_seg_head_fp_workspace_bytes(const svnet_seg_head_fp_params* p)
+{
+    if (!p || p->B < 1 || p->N < 1 || p->Kc < 1 || p->C8 < 1 || p->C9 < 1 || p->C10 < 1 || p->parts < 1) return 0;
+    seg_fp_plan pl;
+    return make_fp_plan(p, &pl) ? pl.total : 0;
+}
+
+extern "C" int svnet_seg_head_fp_fwd(const svnet_seg_head_fp_params* p, void* workspace, size_t workspace_bytes, void* stream)
+{
+    SV_REQUIRE(p && p->logits && p->glob && p->sv.s && p->sv.v && p->Wz1 && p->W8 && p->bn8_a && p->bn8_c && p->W9 && p->bn9_a &&
+                   p->bn9_c && p->W10 && p->bn10_a && p->bn10_c && p->W11,
+               "svnet_seg_head_fp_fwd: null pointer");
+    SV_REQUIRE(p->B >= 0 && p->N >= 1 && p->Kc >= 1 && p->ldg >= p->Kc && p->sv.Cs >= 1 && p->sv.Cv >= 1 && p->C8 >= 1 && p->C9 >= 1 &&
+                   p->C10 >= 1 && p->parts >= 1,
+               "svnet_seg_head_fp_fwd: bad shape");
+    if (p->B == 0) return SVNET_OK;
+    seg_fp_plan pl;
+    SV_REQUIRE(make_fp_plan(p, &pl), "svnet_seg_head_fp_fwd: conv8's per-point linear is not covered by the tensor-core linear (svnet_linear_workspace_bytes)");
+    SV_REQUIRE(workspace && workspace_bytes >= pl.total && !(reinterpret_cast<uintptr_t>(workspace) & 15),
+               "svnet_seg_head_fp_fwd: workspace too small (svnet_seg_head_fp_workspace_bytes) or misaligned");
+    unsigned char* ws = static_cast<unsigned char*>(workspace);
+    cudaStream_t st = sv_stream(stream);
+    const int Kp = p->sv.Cs + 3 * p->sv.Cv;
+    float* u = reinterpret_cast<float*>(ws + pl.u);
+    float* cterm = reinterpret_cast<float*>(ws + pl.cterm);
+    float* hA = reinterpret_cast<float*>(ws + pl.hA);
+    float* hB = reinterpret_cast<float*>(ws + pl.hB);
+    void* lws = ws + pl.lws;
+    // svfuse1: u = [s | v2s(v)] per point
+    int rc = svnet_rows_prep(&p->sv, (long)p->B * p->N, p->Wz1, nullptr, nullptr, nullptr, u, Kp, nullptr, nullptr, nullptr, nullptr, stream);
+    if (rc != SVNET_OK) return rc;
+    svnet_gemm_params g[5];
+    fp_linears(p, u, cterm, hA, hB, g);
+    for (int i = 0; i < 5; ++i) {
+        if (i == 1) {
+            // conv8 adds the per-cloud term g[0] wrote (row r of the point table belongs to cloud r / N)
+            rc = svnet_linear_tc3_rowadd(&g[i], cterm, p->N, p->C8, lws, pl.lws_bytes, st);
+            if (rc < 0) return rc;
+            SV_REQUIRE(rc == 1, "svnet_seg_head_fp_fwd: conv8's tensor-core linear not taken");
+        } else {
+            // as the layer-by-layer path: the tensor-core linear where its workspace query covers the layer
+            const size_t b = svnet_linear_workspace_bytes(&g[i]);
+            rc = svnet_linear_rows_ws(&g[i], b ? lws : nullptr, b, stream);
+            if (rc != SVNET_OK) return rc;
+        }
+    }
+    seg_transpose_kernel<<<dim3(sv_cdiv(p->N, 32), sv_cdiv(p->parts, 32), p->B), 256, 0, st>>>(hB, p->parts, p->N, p->logits);
+    SV_CHECK_LAUNCH("svnet_seg_head_fp_fwd(transpose)");
     return SVNET_OK;
 }

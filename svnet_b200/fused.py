@@ -40,12 +40,14 @@ def native_forward(model, kind, x, extra=None):
     (``_Cached``: rebuilt after load_state_dict / .to(); nn.DataParallel replicas share their source's handles) and makes
     the same library calls as the Python path below -- identical bits -- without Python between the kernels: an eager
     ``model(data)``, which is how the reference's eval loops call it (main_cls_dgcnn.py:238), is no longer bound by the
-    host's launch rate (B = 32: 1.72 -> 1.07 ms)."""
+    host's launch rate (B = 32: 1.72 -> 1.07 ms).  Covered: k = 20, and k = 40 for the binary models and both part-segmentation
+    models."""
     if not NATIVE_FORWARD or not x.is_cuda or x.dtype != torch.float32 or x.dim() != 3 or x.shape[1] != 3:
         return None
     B, _, N = x.shape
     k, binary = model.k, bool(model.binary)
-    if B < 1 or N < 64 or N > 4096 or not (k == 20 or (binary and k == 40)) or (kind == "SV_DGCNN_PSEG" and not binary):
+    pseg = kind == "SV_DGCNN_PSEG"
+    if B < 1 or N < 64 or N > 4096 or not (k == 20 or (k == 40 and (binary or pseg))):
         return None
     if x.device.index != torch.cuda.current_device():
         with torch.cuda.device(x.device):
@@ -56,11 +58,17 @@ def native_forward(model, kind, x, extra=None):
     for blk in (model.conv2, model.conv3, model.conv4):
         if covered(blk.in_dims[0] // 2, blk.in_dims[1] // 2, blk.out_dims[0], blk.out_dims[1], k) == 0:
             return None
+    # ... and the full-precision part-segmentation head's per-point conv8 (svfuse1's Cs + 3Cv channels -> C8), which carries
+    # the per-cloud term, on the tensor-core fp linear (SVNET_LINEAR_TC=0 takes it off); its other linears take either kernel
+    if pseg and not binary:
+        cs, cv = model.conv5.in_dims
+        if nv.linear_tc_bytes(cs + 3 * cv, model.conv8[0].out_channels) == 0:
+            return None
     from .native_model import NativeModel
     names = [n for n, t in model.state_dict().items() if t.dtype == torch.float32] if "_sv_native_names" not in model.__dict__ \
         else model.__dict__["_sv_native_names"]
     model.__dict__["_sv_native_names"] = names
-    ncls = model.linear3.out_features if kind == "SV_DGCNN_CLS" else model.conv11.out_channels
+    ncls = model.conv11.out_channels if pseg else model.linear3.out_features
 
     def build():
         from .sv_layers import _resolve

@@ -1,7 +1,7 @@
 """The whole-model C entry (include/svnet_b200.h: svnet_model_create / _forward / _destroy) behind a Python callable --
 what a C or C++ host would do with the library, spelled out: build the handle from a checkpoint's tensors once, then
-`forward` with caller-owned scratch.  Covered: SV_DGCNN_CLS, binary (k = 20 / 40) or full precision (k = 20), and the binary
-SV_DGCNN_PSEG (`native(batch, label_one_hot)` -> (B, parts, N)); 64 <= N <= 4096.
+`forward` with caller-owned scratch.  Covered: SV_DGCNN_CLS, binary (k = 20 / 40) or full precision (k = 20), and
+SV_DGCNN_PSEG, binary or full precision (k = 20 / 40; `native(batch, label_one_hot)` -> (B, parts, N)); 64 <= N <= 4096.
 
     native = svnet_b200.NativeModel("SV_DGCNN_CLS", checkpoint["state_dict"], k=20, binary=True, num_class=40)
     logits = native(batch)                     # (B, 3, N) float32 CUDA -> (B, num_class); bit-identical to the nn.Module
@@ -35,11 +35,14 @@ class NativeModel:
                 if key not in self._ws:
                     nbytes = nv.model_seg_workspace_bytes(self._h, B, N)
                     if nbytes == 0:
-                        raise ValueError("shape (B=%d, N=%d) is not covered by svnet_model_forward_seg (64 <= N <= 4096)" % (B, N))
+                        raise ValueError("shape (B=%d, N=%d) is not covered by svnet_model_forward_seg (64 <= N <= 4096; a full-precision "
+                                         "model also needs the tensor-core linear for its head's conv8)" % (B, N))
                     self._ws[key] = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
                 logits = torch.empty((B, self.num_class, N), dtype=torch.float32, device=x.device)
                 nv.model_forward_seg(self._h, x.contiguous(), label.reshape(B, -1).contiguous().float(), logits, self._ws[key])
-                nv.LAUNCHES[0] += 60 * self._sub_batches(B, N) - 1     # kernels behind the one call (per sub-batch: trunk 24, conv5 / conv6 branch 18, head 11, ...)
+                if self.binary:       # kernels behind the one call (per sub-batch: trunk 24, conv5 / conv6 branch 18, head 11, ...)
+                    nv.LAUNCHES[0] += 60 * self._sub_batches(B, N) - 1
+                # the full-precision model's call is counted as one launch: its kernel count is not derived here
             return logits
         with torch.cuda.device(x.device):
             key = (B, N)

@@ -10,6 +10,9 @@ row-major (B*N, C) tables:
             ``repeat(1, 1, num_points)`` of :118): their sign words and popcounts are reduced once per
             cloud and enter the per-point popcount linear as an integer offset      (:117-121)
     conv9/10 binary conv + BN + leaky, conv11 fp                                       (:123-126)
+The full-precision head is one call as well (svnet_seg_head_fp_fwd): conv8's per-cloud 1600 columns are one linear over the
+B clouds, added per point in the epilogue of the per-point linear over svfuse1's 544 channels (on the three-plane
+tensor-core fp linear); conv9 .. conv11 take the kernel the layer-by-layer calls take.  SVNET_SEG_HEAD_CALL=0 runs both heads layer by layer (the fp one over the (B*N, 2144) table).
 """
 import os
 
@@ -97,7 +100,9 @@ class SV_DGCNN_PSEG(_Cached, nn.Module):
         return chunked(lambda xc, lc: self._forward(xc, lc, forced_idx, record), x, (l,), hooks=hooks)
 
     def _forward(self, x, l, forced_idx=None, record=None):
-        """x (B,3,N), l (B,16) one-hot -> per-point part logits (B, num_part, N)."""
+        """x (B,3,N), l (B,16) one-hot -> per-point part logits (B, num_part, N).  The calls csrc/model.cu's
+        svnet_model_forward_seg makes in C (binary or full precision), so the two paths give the same bits; with ``record``
+        (test hooks) the head runs layer by layer."""
         _inference_only(self)
         B, _, N = x.shape
         R = B * N
@@ -105,9 +110,11 @@ class SV_DGCNN_PSEG(_Cached, nn.Module):
         s_cat, v_cat = dgcnn_trunk(self, x, forced_idx, record)
         C5s, C5v = self.conv5.out_dims
         fuse3 = 3 * C5v <= 512             # svfuse3 + max pooling without the (R, 1016) table (svnet_svfuse_pool)
-        # svfuse1's output only feeds conv8: a binary conv8 takes its sign words straight from (s_cat, v_cat)
+        # svfuse1's output only feeds conv8: a binary conv8 takes its sign words straight from (s_cat, v_cat), the fp head call
+        # writes the rows into its own scratch
         lean_fine = self.binary and record is None
-        x_fine = None if lean_fine else self.svfuse1.forward_rows(s_cat, v_cat)[0]          # (R, 544)
+        fp_head = not self.binary and record is None and SEG_HEAD_CALL
+        x_fine = None if (lean_fine or fp_head) else self.svfuse1.forward_rows(s_cat, v_cat)[0]          # (R, 544)
         sv_in = sv_bits = aux = None
         if lean_fine:
             # conv8's per-point sign words depend on the trunk only: they run on a side stream next to the global
@@ -181,6 +188,17 @@ class SV_DGCNN_PSEG(_Cached, nn.Module):
             h = self.conv8[0].forward_rows(None, bn=self.conv8.bn_folded(), act=nv.ACT_LEAKY, cloud=glob, rows_per_cloud=N,
                                            sv_in=sv_in, sv_bits=sv_bits)
         else:
+            if fp_head:
+                W11 = self.conv11.weight.detach()[:, :, 0]
+                # conv8 .. conv11 as one C-ABI call (csrc/seg_head.cu): conv8's per-cloud part of the (R, 2144) input once per
+                # cloud, the per-point part over svfuse1's 544 channels; None when conv8 is off the tensor-core linear
+                layers = [(c.weight2d(), seq.bn_folded()) for c, seq in ((self.conv8[0], self.conv8), (self.conv9[0], self.conv9),
+                                                                          (self.conv10[0], self.conv10))]
+                y = nv.seg_head_fp_fwd(nv.view_of(s_cat, v_cat), B, N, self.svfuse1.v2s.wz()[0], glob, layers,
+                                       W11 if W11.is_contiguous() else W11.contiguous())
+                if y is not None:
+                    return y
+                x_fine = self.svfuse1.forward_rows(s_cat, v_cat)[0]
             h = self.conv8[0].forward_rows(x_fine, bn=self.conv8.bn_folded(), act=nv.ACT_LEAKY, cloud=glob, rows_per_cloud=N)
         h = self.conv9[0].forward_rows(h, bn=self.conv9.bn_folded(), act=nv.ACT_LEAKY)
         h = self.conv10[0].forward_rows(h, bn=self.conv10.bn_folded(), act=nv.ACT_LEAKY)
