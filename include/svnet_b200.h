@@ -300,7 +300,7 @@ typedef struct {
 } svnet_gemm_params;
 int svnet_linear_rows(const svnet_gemm_params* p, void* stream);
 /* With svnet_linear_workspace_bytes(p) bytes of caller-owned scratch (16-byte aligned) a plain fp32 linear
- * (G == 1, no sign_w / vbn / gate, 32 <= N <= 512, 32 <= K <= 4096; chosen by (K, N) only, never by the row count) runs on the tcgen05 tensor cores with
+ * (G == 1, no sign_w / vbn / gate / c4, 32 <= N <= 512, 32 <= K <= 4096; chosen by (K, N) only, never by the row count) runs on the tcgen05 tensor cores with
  * both operands split exactly into three bf16 planes (six plane products, fp32 accumulation in tensor memory:
  * fp32-level accuracy, different summation order -> tolerance-level, csrc/gemm_tc3.cu).  0 bytes: not covered,
  * svnet_linear_rows_ws then behaves as svnet_linear_rows. */

@@ -149,6 +149,7 @@ struct tc3_args {
     const float* A;
     long lda, rows;
     int K, N, MT, NKC;       // MT = channel tiles handled by one CTA (blockIdx.y selects the group)
+    int MT_total;            // channel tiles in the packed weights: the last group may hold fewer than MT
     const unsigned char* Wtc;
     const float* colscale;
     const float* bias;
@@ -164,7 +165,11 @@ struct tc3_args {
 __global__ void __launch_bounds__(NTH, 1) gemm_tc3_kernel(tc3_args p)
 {
     extern __shared__ __align__(1024) unsigned char smraw[];
-    const int NKC = p.NKC, MT = p.MT;
+    const int NKC = p.NKC;
+    const int mt0 = blockIdx.y * p.MT;                           // first channel tile of this CTA
+    // tiles of this CTA: with an odd tile count the last group has one (N = 257..384 at two tiles per CTA); a tile
+    // past the last would stream weight chunks from beyond the end of the workspace
+    const int MT = min(p.MT, p.MT_total - mt0);
     unsigned char* Bs = smraw;                                   // activations: 2 chunks (double buffer)
     unsigned char* Ring = Bs + 2 * CHUNK_BYTES;                  // weight chunks
     uint64_t* bars = reinterpret_cast<uint64_t*>(Ring + (size_t)STAGES * CHUNK_BYTES);
@@ -177,7 +182,6 @@ __global__ void __launch_bounds__(NTH, 1) gemm_tc3_kernel(tc3_args p)
 
     const int tid = threadIdx.x, lane = tid & 31, warp = sv_warp_id();
     const long r0 = (long)blockIdx.x * TR;
-    const int mt0 = blockIdx.y * MT;         // first channel tile of this CTA
 
     if (tid == 0) {
         for (int s = 0; s < STAGES; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
@@ -332,7 +336,7 @@ bool tc3_plan(const svnet_gemm_params* p, int* MT, int* NKC, size_t* wbytes, siz
 {
     const char* on = getenv("SVNET_LINEAR_TC");
     if (on && on[0] == '0') return false;
-    if (p->G != 1 || p->sign_w || p->vbn || p->gate) return false;
+    if (p->G != 1 || p->sign_w || p->vbn || p->gate || p->c4) return false;     // c4: the float4 table is not this layout
     // The choice must not depend on the number of rows: this path rounds differently from the CUDA-core chain,
     // and a cloud's result has to be the same bits whatever batch (or batch shard) it is part of.
     if (p->M < 1 || p->K < 32 || p->K > 4096 || p->N < 32 || p->N > MT_MAX * TCH) return false;
@@ -370,7 +374,7 @@ int svnet_linear_tc3_rowadd(const svnet_gemm_params* p, const float* rowadd, lon
     // tiles one channel tile per CTA so that more SMs take part (the activations are staged per CTA)
     const int row_tiles = sv_cdiv(p->M, TR);
     const int mt_per_cta = row_tiles >= 64 ? (MT < 2 ? MT : 2) : 1;
-    a.A = p->A; a.lda = p->lda_g; a.rows = p->M; a.K = p->K; a.N = p->N; a.MT = mt_per_cta; a.NKC = NKC;
+    a.A = p->A; a.lda = p->lda_g; a.rows = p->M; a.K = p->K; a.N = p->N; a.MT = mt_per_cta; a.MT_total = MT; a.NKC = NKC;
     a.Wtc = static_cast<const unsigned char*>(workspace);
     a.colscale = p->colscale; a.bias = p->bias; a.bn_a = p->bn_a; a.bn_c = p->bn_c; a.act = p->act;
     a.C = p->C; a.ldc = p->ldc_g;
