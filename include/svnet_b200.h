@@ -73,8 +73,18 @@ const char* svnet_last_error(void);
 /* sign(W) bit-planes for a binarised Linear/Conv1d weight (sv_layers.py:43-45,70).
  * W [rows][ldw] (first K columns used) -> bits_t [ceil(K/32)][rows] (word-major, bit b of word w
  * = (W[row][32w+b] > 0)).  *zero_count (device int) receives the number of exactly-zero weights
- * (sign(0)=0 is not representable in one plane; callers must reject > 0). */
+ * (sign(0)=0 is not representable in one plane: with a count > 0 the consumers need the non-zero
+ * plane of svnet_pack_sign_nz as well). */
 int svnet_pack_sign(const float* W, int rows, int K, int ldw, uint32_t* bits_t, int* zero_count, void* stream);
+
+/* The same sign plane plus the non-zero plane of a ternary weight (torch.sign(W) in {-1, 0, +1}):
+ * nz_t [ceil(K/32)][rows], bit b of word w = (W[row][32w+b] != 0), K tail 0.  -0.0 counts as zero
+ * (as torch.sign(-0.0) == 0), subnormal weights as +-1.  bits_t and *zero_count as svnet_pack_sign.
+ * The consumers below take nz_t as `W1nz` through their *_nz entry points; NULL there means every
+ * weight is +-1 (the plain entry points are those calls with NULL), so a caller keeps a plane only
+ * where the zero count of its slice is > 0. */
+int svnet_pack_sign_nz(const float* W, int rows, int K, int ldw, uint32_t* bits_t, uint32_t* nz_t, int* zero_count,
+                       void* stream);
 
 /* eval-mode BatchNorm1d as y = x*a + c (torch.nn.BatchNorm1d with running stats; sv_layers.py:84,166):
  * a = w/sqrt(var+eps), c = b - mean*a. */
@@ -206,6 +216,11 @@ typedef struct {
                                 * input vectors; one svnet_linear_rows call with `c4` set produces it */
 } svnet_edge_params;
 int svnet_svblock_edge_fwd(const svnet_edge_params* p, void* stream);
+/* Binary layers with ternary weights: W1nz [Kw][Cout] is the non-zero plane of conv.linear1.weight (svnet_pack_sign_nz)
+ * or NULL (every weight +-1: svnet_svblock_edge_fwd).  y_o = scale1_o * sum over words of
+ * (popc(m & z_o) - 2 popc((a ^ w_o) & m & z_o)).  The tensor-core kernel takes its zeros from W1tc; otherwise a call with a
+ * plane runs the generic kernel (the shape-specialised CUDA-core kernels are +-1 only). */
+int svnet_svblock_edge_fwd_nz(const svnet_edge_params* p, const uint32_t* W1nz, void* stream);
 
 /* Tensor-core variant of the binary edge layers (sv_layers.py:36-49 on sv_util.py:90-116's edge features).
  * svnet_edge_tc_weight_bytes() is 0 for shapes / k the kernel does not cover (covered: the six edge-layer shapes of
@@ -270,6 +285,13 @@ int svnet_binlinear_rows_ws(const uint32_t* bits, const uint32_t* mask, const in
                             const uint32_t* W1b, int Cout, const float* scale, const float* bias, const float* bn_a,
                             const float* bn_c, int act, const int32_t* cloud_dot, long rows_per_cloud, float* out,
                             int ldo, int32_t* out_i32, void* workspace, size_t workspace_bytes, void* stream);
+/* svnet_binlinear_rows_ws with ternary weights: W1nz [Kw][Cout] non-zero plane of the weight (svnet_pack_sign_nz) or NULL
+ * (every weight +-1, the calls above).  dot = sum over words of popc(m & z_o) - 2 popc((a ^ w_o) & m & z_o): the count of
+ * non-zero products depends on (row, channel) and replaces nvalid_r.  Same kernels, same tensor-core coverage. */
+int svnet_binlinear_rows_nz(const uint32_t* bits, const uint32_t* mask, const int32_t* nvalid, long rows, int K,
+                            const uint32_t* W1b, const uint32_t* W1nz, int Cout, const float* scale, const float* bias,
+                            const float* bn_a, const float* bn_c, int act, const int32_t* cloud_dot, long rows_per_cloud,
+                            float* out, int ldo, int32_t* out_i32, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Binarised Linear -> BN -> LeakyReLU fused with the per-cloud max / mean over the rows (tensor-core path
  * only): the (rows, Cout) activation is never written.  SV_DGCNN_CLS pools conv5's scalar output right away
@@ -280,6 +302,11 @@ int svnet_binlinear_pool_ws(const uint32_t* bits, const uint32_t* mask, long row
                             const float* scale, const float* bn_a, const float* bn_c, long rows_per_cloud,
                             float* max_out, float* mean_out, int ldo, void* workspace, size_t workspace_bytes,
                             void* stream);
+/* The same with ternary weights: W1nz as in svnet_binlinear_rows_nz (NULL: svnet_binlinear_pool_ws). */
+int svnet_binlinear_pool_nz(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b,
+                            const uint32_t* W1nz, int Cout, const float* scale, const float* bn_a, const float* bn_c,
+                            long rows_per_cloud, float* max_out, float* mean_out, int ldo, void* workspace,
+                            size_t workspace_bytes, void* stream);
 
 /* Generic fp32 linear over (grouped) rows: C[m][n] = epi(sum_k A[m][k] * W[n][k]), sequential fmaf
  * chain over k (== oracle order).  Row m lives at A + (m / G)*lda_g + (m % G)*lda_x; same for C.
@@ -330,6 +357,10 @@ typedef struct {
     float* out; int ldo;
 } svnet_head_params;
 int svnet_head_fwd(const svnet_head_params* p, void* stream);
+/* Binary layers with ternary weights: W1nz[l] is the non-zero plane [Kw][Cout] of layer l's weight (svnet_pack_sign_nz) or
+ * NULL (+-1 weights); W1nz itself may be NULL (svnet_head_fwd).  A call with any plane reads the sign planes from global
+ * memory instead of prefetching them into shared memory. */
+int svnet_head_fwd_nz(const svnet_head_params* p, const uint32_t* const W1nz[3], void* stream);
 
 /* Part-segmentation head as one call (sv_dgcnn_partseg.py:112-126): conv8 over [per-cloud channels | svfuse1(s_cat, v_cat)]
  * -> conv9 -> conv10 (binarised Conv1d + BN + LeakyReLU, sv_layers.py:64-78) -> conv11 (fp Conv1d) -> logits in the
@@ -356,6 +387,10 @@ typedef struct {
 } svnet_seg_head_params;
 size_t svnet_seg_head_workspace_bytes(const svnet_seg_head_params* p);
 int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspace, size_t workspace_bytes, void* stream);
+/* The same with ternary weights: non-zero planes (svnet_pack_sign_nz) of W8c, W8p, W9 and W10, each NULL when that plane's
+ * weights are all +-1 (all NULL: svnet_seg_head_fwd).  Same workspace. */
+int svnet_seg_head_fwd_nz(const svnet_seg_head_params* p, const uint32_t* W8c_nz, const uint32_t* W8p_nz, const uint32_t* W9_nz,
+                          const uint32_t* W10_nz, void* workspace, size_t workspace_bytes, void* stream);
 
 /* The same head of the full-precision model (binary = False: plain Conv1d weights, no beta / scale) as one call.  conv8's
  * input is [glob[b] repeated over the points | svfuse1(s_cat, v_cat)]; its per-cloud part W8[:, :Kc] glob[b] is computed

@@ -29,6 +29,8 @@ EXPORTS = [
     "svnet_edge_fp_tc_weight_bytes", "svnet_edge_fp_tc_pack_w", "svnet_seg_head_fwd", "svnet_seg_head_workspace_bytes",
     "svnet_model_create", "svnet_model_workspace_bytes", "svnet_model_forward", "svnet_model_destroy",
     "svnet_model_seg_workspace_bytes", "svnet_model_forward_seg", "svnet_seg_head_fp_workspace_bytes", "svnet_seg_head_fp_fwd",
+    "svnet_pack_sign_nz", "svnet_binlinear_rows_nz", "svnet_binlinear_pool_nz", "svnet_head_fwd_nz", "svnet_svblock_edge_fwd_nz",
+    "svnet_seg_head_fwd_nz",
 ]
 
 
@@ -188,7 +190,7 @@ def view_of(s, v, Cs=None, Cv=None):
 # thin wrappers (shapes validated again on the C side)
 # ------------------------------------------------------------------------------------------------
 def pack_sign(W2d):
-    """W (rows, K) float -> bits_t (Kw, rows) int32 (word-major); raises on exact-zero weights."""
+    """W (rows, K) float -> bits_t (Kw, rows) int32 (word-major); raises on exact-zero weights (see pack_sign_nz)."""
     W2d = _dev(W2d)
     assert W2d.dim() == 2 and W2d.stride(1) == 1
     rows, K = W2d.shape
@@ -199,6 +201,20 @@ def pack_sign(W2d):
     if int(zc.item()) != 0:
         raise NotImplementedError("binarised weight contains exact zeros (sign(0)=0 plane not supported)")
     return bits
+
+
+def pack_sign_nz(W2d):
+    """W (rows, K) float -> (bits_t, nz_t): the sign plane and, when W holds an exact zero (-0.0 included), its non-zero
+    plane (Kw, rows) int32; nz_t is None for a zero-free W, whose consumers then run their +-1 kernels."""
+    W2d = _dev(W2d)
+    assert W2d.dim() == 2 and W2d.stride(1) == 1
+    rows, K = W2d.shape
+    bits = torch.empty(((K + 31) // 32, rows), dtype=torch.int32, device=W2d.device)
+    nz = torch.empty_like(bits)
+    zc = torch.zeros(1, dtype=torch.int32, device=W2d.device)
+    _call("svnet_pack_sign_nz", _ptr(W2d), c_int(rows), c_int(K), c_int(W2d.stride(0)), _ptr(bits), _ptr(nz), _ptr(zc),
+          _stream())
+    return bits, (nz if int(zc.item()) != 0 else None)
 
 
 def fold_bn(bn):
@@ -274,8 +290,12 @@ def edge_xyz_fwd(params):
     _call("svnet_edge_xyz_fwd", ctypes.byref(params), _stream())
 
 
-def svblock_edge_fwd(params):
-    _call("svnet_svblock_edge_fwd", ctypes.byref(params), _stream())
+def svblock_edge_fwd(params, W1nz=None):
+    """``W1nz``: non-zero plane of a binary layer's ternary linear1 weight (pack_sign_nz), or None."""
+    if W1nz is None:
+        _call("svnet_svblock_edge_fwd", ctypes.byref(params), _stream())
+    else:
+        _call("svnet_svblock_edge_fwd_nz", ctypes.byref(params), _ptr(W1nz), _stream())
 
 
 def edge_tc_weight_bytes(Cs, Cv, Cout, Cvo, k):
@@ -310,7 +330,8 @@ def edge_fp_tc_pack_w(W1, Cs, Cv, nbytes):
 
 def seg_head_fwd(view, B, N, Wz1, zscale1, glob, layers, W11, sv_bits=None):
     """svnet_seg_head_fwd: conv8 -> conv9 -> conv10 -> conv11 of SV_DGCNN_PSEG in one call.  ``layers`` = three dicts
-    (beta, bits (conv8: (bits of the per-cloud part, bits of the per-point part)), scale, bn (a, c), Cout);
+    (beta, bits (conv8: (bits of the per-cloud part, bits of the per-point part)), nz (the same for the non-zero planes,
+    None where the weights are +-1), scale, bn (a, c), Cout);
     ``sv_bits`` = conv8's per-point (bits, mask, nvalid) computed ahead of time, or None.  Returns (B, parts, N)."""
     glob, W11 = _dev(glob), _dev(W11)
     p = SegHeadParams()
@@ -331,7 +352,11 @@ def seg_head_fwd(view, B, N, Wz1, zscale1, glob, layers, W11, sv_bits=None):
     p.logits = out.data_ptr()
     nbytes = int(lib().svnet_seg_head_workspace_bytes(ctypes.byref(p)))
     ws = torch.empty(nbytes, dtype=torch.uint8, device=glob.device)
-    _call("svnet_seg_head_fwd", ctypes.byref(p), _ptr(ws), ctypes.c_size_t(nbytes), _stream())
+    nzs = list(l8.get("nz") or (None, None)) + [l9.get("nz"), l10.get("nz")]
+    if all(z is None for z in nzs):
+        _call("svnet_seg_head_fwd", ctypes.byref(p), _ptr(ws), ctypes.c_size_t(nbytes), _stream())
+    else:
+        _call("svnet_seg_head_fwd_nz", ctypes.byref(p), *[_ptr(z) for z in nzs], _ptr(ws), ctypes.c_size_t(nbytes), _stream())
     LAUNCHES[0] += 11        # kernels behind the one call (sign-packs, binarised linears, GEMM, transpose)
     return out
 
@@ -420,7 +445,8 @@ def rows_prep(view, rows, Wz=None, zscale=None, beta=None, u_out=None, ldu=0, z_
 
 
 def binlinear_rows(bits, mask, nvalid, K, W1b, Cout, scale=None, bias=None, bn=None, act=ACT_NONE, cloud_dot=None,
-                   rows_per_cloud=1, out=None, ldo=None, out_i32=False):
+                   rows_per_cloud=1, out=None, ldo=None, out_i32=False, W1nz=None):
+    """``W1nz``: non-zero plane of ternary weights (pack_sign_nz), or None (+-1 weights)."""
     rows = bits.shape[0]
     res_i32 = None
     if out_i32:
@@ -432,10 +458,10 @@ def binlinear_rows(bits, mask, nvalid, K, W1b, Cout, scale=None, bias=None, bn=N
     # scratch for the expanded weights of the tensor-core path; 0 bytes -> popcount kernel
     nbytes = int(lib().svnet_binlinear_workspace_bytes(c_long(rows), c_int(K), c_int(Cout)))
     ws = torch.empty(nbytes, dtype=torch.uint8, device=bits.device) if nbytes > 0 else None
-    _call("svnet_binlinear_rows_ws", _ptr(bits), _ptr(mask), _ptr(nvalid), c_long(rows), c_int(K), _ptr(W1b),
-                                         c_int(Cout), _ptr(scale), _ptr(bias), _ptr(bn_a), _ptr(bn_c), c_int(act),
-                                         _ptr(cloud_dot), c_long(rows_per_cloud), _ptr(out), c_int(ldo or 0),
-                                         _ptr(res_i32), _ptr(ws), ctypes.c_size_t(nbytes), _stream())
+    name, wargs = ("svnet_binlinear_rows_ws", (_ptr(W1b),)) if W1nz is None else ("svnet_binlinear_rows_nz", (_ptr(W1b), _ptr(W1nz)))
+    _call(name, _ptr(bits), _ptr(mask), _ptr(nvalid), c_long(rows), c_int(K), *wargs, c_int(Cout), _ptr(scale), _ptr(bias),
+          _ptr(bn_a), _ptr(bn_c), c_int(act), _ptr(cloud_dot), c_long(rows_per_cloud), _ptr(out), c_int(ldo or 0),
+          _ptr(res_i32), _ptr(ws), ctypes.c_size_t(nbytes), _stream())
     if nbytes > 0:
         LAUNCHES[0] += 1
     return res_i32 if out_i32 else out
@@ -445,12 +471,14 @@ def binlinear_pool_workspace(rows, K, Cout, rows_per_cloud):
     return int(lib().svnet_binlinear_pool_workspace_bytes(c_long(rows), c_int(K), c_int(Cout), c_long(rows_per_cloud)))
 
 
-def binlinear_pool(bits, mask, K, W1b, Cout, scale, bn, rows_per_cloud, max_out, mean_out, ldo):
-    """Binarised Linear -> BN -> LeakyReLU -> per-cloud max / mean, fused (tensor-core path only)."""
+def binlinear_pool(bits, mask, K, W1b, Cout, scale, bn, rows_per_cloud, max_out, mean_out, ldo, W1nz=None):
+    """Binarised Linear -> BN -> LeakyReLU -> per-cloud max / mean, fused (tensor-core path only); ``W1nz`` as in
+    binlinear_rows."""
     rows = bits.shape[0]
     nbytes = binlinear_pool_workspace(rows, K, Cout, rows_per_cloud)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=bits.device)
-    _call("svnet_binlinear_pool_ws", _ptr(bits), _ptr(mask), c_long(rows), c_int(K), _ptr(W1b), c_int(Cout), _ptr(scale),
+    name, wargs = ("svnet_binlinear_pool_ws", (_ptr(W1b),)) if W1nz is None else ("svnet_binlinear_pool_nz", (_ptr(W1b), _ptr(W1nz)))
+    _call(name, _ptr(bits), _ptr(mask), c_long(rows), c_int(K), *wargs, c_int(Cout), _ptr(scale),
           _ptr(bn[0]), _ptr(bn[1]), c_long(rows_per_cloud), _ptr(max_out), _ptr(mean_out), c_int(ldo), _ptr(ws),
           ctypes.c_size_t(nbytes), _stream())
     LAUNCHES[0] += 2
@@ -522,7 +550,8 @@ def pool_rows(x, ld, C, B, rows, want_max=True, want_mean=False, max_out=None, m
 
 
 def head_fwd(x2d, layers):
-    """layers: list of dicts(Cout, W1b, beta, W, sign_w, scale, bias, bn=(a, c), act) -> (B, Cout_last)."""
+    """layers: list of dicts(Cout, W1b, W1nz (non-zero plane or None), beta, W, sign_w, scale, bias, bn=(a, c), act)
+    -> (B, Cout_last)."""
     B, K0 = x2d.shape
     p = HeadParams()
     p.x, p.ldx, p.K0, p.B, p.nlayers = _dev(x2d).data_ptr(), x2d.stride(0), K0, B, len(layers)
@@ -540,7 +569,12 @@ def head_fwd(x2d, layers):
         hl.act = L.get("act", ACT_NONE)
     out = torch.empty((B, layers[-1]["Cout"]), dtype=torch.float32, device=x2d.device)
     p.out, p.ldo = out.data_ptr(), out.shape[1]
-    _call("svnet_head_fwd", ctypes.byref(p), _stream())
+    nzs = [L.get("W1nz") for L in layers]
+    if all(z is None for z in nzs):
+        _call("svnet_head_fwd", ctypes.byref(p), _stream())
+    else:
+        arr = (c_void_p * 3)(*[z.data_ptr() if z is not None else None for z in nzs + [None] * (3 - len(nzs))])
+        _call("svnet_head_fwd_nz", ctypes.byref(p), arr, _stream())
     return out
 
 

@@ -1,7 +1,8 @@
 // Binarised Linear / Conv1d over packed rows on the tcgen05 tensor cores
 // (reference models/sv_layers.py:29-53, :64-78: y = sign(x + beta) . sign(W)^T * scale).
 // Same contract as rows.cu:binlinear_rows_kernel -- the dot product of ternary activations
-// {-1, 0, +1} (sign / zero-mask words) with +-1 weights is an exact integer -- but the products run as
+// {-1, 0, +1} (sign / zero-mask words) with +-1 (or, with a non-zero plane, ternary) weights is an exact integer --
+// but the products run as
 // bf16 UMMAs with fp32 accumulation in tensor memory: every operand value is exactly representable and
 // every partial sum is an integer below 2^24, so the result is bit-identical to the XNOR/popcount kernel
 // (which is bound by the quarter-rate POPC pipe).
@@ -117,9 +118,11 @@ __device__ __forceinline__ uint4 expand8(uint32_t pos, uint32_t nz)
     return make_uint4(w[0], w[1], w[2], w[3]);
 }
 
-// sign-bit words W1b [Kw][Cout] -> Wtc [MT][NKC][8 k-blocks][128 channels][8 bf16] (+-1, zero padded)
+// sign-bit words W1b [Kw][Cout] -> Wtc [MT][NKC][8 k-blocks][128 channels][8 bf16] (+-1, zero padded).
+// TERN: W1nz [Kw][Cout] is the non-zero plane of ternary weights; a zero weight is an exact bf16 0.
+template <bool TERN>
 __global__ void binlinear_pack_w_kernel(const uint32_t* __restrict__ W1b, int Kw, int K, int Cout, int MT, int NKC,
-                                        uint4* __restrict__ Wtc)
+                                        uint4* __restrict__ Wtc, const uint32_t* __restrict__ W1nz)
 {
     const int total = MT * NKC * 8 * TCH;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
@@ -130,7 +133,8 @@ __global__ void binlinear_pack_w_kernel(const uint32_t* __restrict__ W1b, int Kw
             const uint32_t word = __ldg(W1b + (long)(k0 >> 5) * Cout + c);
             pos = (word >> (k0 & 31)) & 0xFFu;
             const int nvalid = min(8, K - k0);
-            nz = (1u << nvalid) - 1u;           // every real weight is +-1 (exact zeros are rejected at pack time)
+            nz = (1u << nvalid) - 1u;           // without a plane every real weight is +-1
+            if (TERN) nz &= (__ldg(W1nz + (long)(k0 >> 5) * Cout + c) >> (k0 & 31)) & 0xFFu;
         }
         Wtc[i] = expand8(pos, nz);
     }
@@ -326,7 +330,18 @@ bool bl_plan(long rows, int K, int Cout, int* MT, int* NKC, size_t* wbytes, size
     return *smem <= 227 * 1024;
 }
 
+// weights -> bf16 operand chunks in the workspace (+-1, or ternary with a non-zero plane)
+void bl_pack_w(const uint32_t* W1b, const uint32_t* W1nz, int Kw, int K, int Cout, int MT, int NKC, void* workspace, cudaStream_t st)
+{
+    const int grid = sv_cdiv((long)MT * NKC * 8 * TCH, 256);
+    if (W1nz)
+        binlinear_pack_w_kernel<true><<<grid, 256, 0, st>>>(W1b, Kw, K, Cout, MT, NKC, static_cast<uint4*>(workspace), W1nz);
+    else
+        binlinear_pack_w_kernel<false><<<grid, 256, 0, st>>>(W1b, Kw, K, Cout, MT, NKC, static_cast<uint4*>(workspace), nullptr);
+}
+
 }  // namespace
+
 
 extern "C" size_t svnet_binlinear_workspace_bytes(long rows, int K, int Cout)
 {
@@ -337,10 +352,10 @@ extern "C" size_t svnet_binlinear_workspace_bytes(long rows, int K, int Cout)
 }
 
 // Returns 1 if handled, 0 if the caller should use the popcount kernel, < 0 on error.
-int svnet_binlinear_tc_dispatch(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b, int Cout,
-                                const float* scale, const float* bias, const float* bn_a, const float* bn_c, int act,
-                                const int32_t* cloud_dot, long rows_per_cloud, float* out, int ldo, int32_t* out_i32,
-                                void* workspace, size_t workspace_bytes, cudaStream_t st)
+int svnet_binlinear_tc_dispatch(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b,
+                                const uint32_t* W1nz, int Cout, const float* scale, const float* bias, const float* bn_a,
+                                const float* bn_c, int act, const int32_t* cloud_dot, long rows_per_cloud, float* out, int ldo,
+                                int32_t* out_i32, void* workspace, size_t workspace_bytes, cudaStream_t st)
 {
     int MT, NKC;
     size_t wb, smem;
@@ -355,8 +370,7 @@ int svnet_binlinear_tc_dispatch(const uint32_t* bits, const uint32_t* mask, long
         if (!lean && !(on && on[0] == '2')) return 0;
     }
     const int Kw = (K + 31) / 32;
-    binlinear_pack_w_kernel<<<sv_cdiv((long)MT * NKC * 8 * TCH, 256), 256, 0, st>>>(W1b, Kw, K, Cout, MT, NKC,
-                                                                                   static_cast<uint4*>(workspace));
+    bl_pack_w(W1b, W1nz, Kw, K, Cout, MT, NKC, workspace, st);
     SV_CHECK_LAUNCH("svnet_binlinear_rows(pack)");
     bl_args a;
     a.bits = bits; a.mask = mask; a.rows = rows; a.Kw = Kw; a.Cout = Cout; a.MT = MT; a.NKC = NKC;
@@ -404,8 +418,8 @@ extern "C" size_t svnet_binlinear_pool_workspace_bytes(long rows, int K, int Cou
     return wb + (size_t)(rows / TR) * 2 * 2 * Cout * sizeof(float);
 }
 
-extern "C" int svnet_binlinear_pool_ws(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b,
-                                       int Cout, const float* scale, const float* bn_a, const float* bn_c,
+extern "C" int svnet_binlinear_pool_nz(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b,
+                                       const uint32_t* W1nz, int Cout, const float* scale, const float* bn_a, const float* bn_c,
                                        long rows_per_cloud, float* max_out, float* mean_out, int ldo, void* workspace,
                                        size_t workspace_bytes, void* stream)
 {
@@ -421,8 +435,7 @@ extern "C" int svnet_binlinear_pool_ws(const uint32_t* bits, const uint32_t* mas
     bl_plan(rows, K, Cout, &MT, &NKC, &wb, &smem);
     cudaStream_t st = sv_stream(stream);
     const int Kw = (K + 31) / 32;
-    binlinear_pack_w_kernel<<<sv_cdiv((long)MT * NKC * 8 * TCH, 256), 256, 0, st>>>(W1b, Kw, K, Cout, MT, NKC,
-                                                                                   static_cast<uint4*>(workspace));
+    bl_pack_w(W1b, W1nz, Kw, K, Cout, MT, NKC, workspace, st);
     SV_CHECK_LAUNCH("svnet_binlinear_pool_ws(pack)");
     bl_args a;
     a.bits = bits; a.mask = mask; a.rows = rows; a.Kw = Kw; a.Cout = Cout; a.MT = MT; a.NKC = NKC;
@@ -438,4 +451,13 @@ extern "C" int svnet_binlinear_pool_ws(const uint32_t* bits, const uint32_t* mas
                                                                              rows_per_cloud, max_out, mean_out, ldo);
     SV_CHECK_LAUNCH("svnet_binlinear_pool_ws(reduce)");
     return SVNET_OK;
+}
+
+extern "C" int svnet_binlinear_pool_ws(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b,
+                                       int Cout, const float* scale, const float* bn_a, const float* bn_c,
+                                       long rows_per_cloud, float* max_out, float* mean_out, int ldo, void* workspace,
+                                       size_t workspace_bytes, void* stream)
+{
+    return svnet_binlinear_pool_nz(bits, mask, rows, K, W1b, nullptr, Cout, scale, bn_a, bn_c, rows_per_cloud, max_out,
+                                   mean_out, ldo, workspace, workspace_bytes, stream);
 }

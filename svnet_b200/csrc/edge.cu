@@ -11,6 +11,8 @@
 //      (torch.sign(0) == 0) -- binary model; or stores q as floats -- fp model.
 //   B. binary: XNOR/popcount linear1, lanes = output channels, accumulating EB edges at a time;
 //      y = scale * (nvalid - 2*popc((a ^ w) & m)); BN affine; LeakyReLU; running max over edges.
+//      Ternary weights (TERN, non-zero plane z staged next to W1b): the count of non-zero products depends on
+//      (edge, channel), y = scale * sum over words of (popc(m & z) - 2*popc((a ^ w) & m & z)).
 //      fp: y = (Ya_j - Ya_i) + Yb_i + W1q q with the per-point tables Ya/Yb.
 //   C. vector branch from the per-point tables P = v W2a^T, Q = v W2b^T:
 //      w = (P_j - P_i) + Q_i; VectorBN; gate; mean over edges.
@@ -32,6 +34,7 @@ struct Smem {
     float* Wz;      // [3][Cve]
     float* beta;    // [K]
     uint32_t* W1b;  // [Kw][Cout]
+    uint32_t* W1z;  // [Kw][Cout] non-zero plane (ternary weights only)
     float* scale1;  // [Cout]
     float* a1;
     float* c1;
@@ -54,24 +57,26 @@ struct Dims {
     size_t shared_floats, warp_floats;
 };
 
-__host__ __device__ inline Dims make_dims(int Cs, int Cv, int k, int Cout, int Cvo, bool binary)
+__host__ __device__ inline Dims make_dims(int Cs, int Cv, int k, int Cout, int Cvo, bool binary, bool tern = false)
 {
     Dims d;
     d.Cs = Cs; d.Cv = Cv; d.Cve = 2 * Cv; d.F = Cs + 3 * Cv; d.K = 2 * Cs + 6 * Cv; d.Kw = (d.K + 31) / 32;
     d.k = k; d.kp = ((k + EB - 1) / EB) * EB; d.Cout = Cout; d.Cvo = Cvo;
-    d.shared_floats = (size_t)3 * d.Cve + d.K + (binary ? (size_t)d.Kw * Cout : 0) + 3 * (size_t)Cout + 2 * (size_t)Cvo + 4;
+    d.shared_floats = (size_t)3 * d.Cve + d.K + (binary ? (size_t)d.Kw * Cout : 0) + (tern ? (size_t)d.Kw * Cout : 0) +
+                      3 * (size_t)Cout + 2 * (size_t)Cvo + 4;
     d.warp_floats = (size_t)d.F * (1 + EG) + EG * 9 + 3 +
                     (binary ? (size_t)2 * d.Kw * d.kp + d.kp : (size_t)EB * 3 * d.Cve) + d.kp;
     return d;
 }
 
-__device__ inline Smem carve(float* base, const Dims& d, bool binary, int warp)
+__device__ inline Smem carve(float* base, const Dims& d, bool binary, int warp, bool tern = false)
 {
     Smem s;
     float* p = base;
     s.Wz = p; p += 3 * d.Cve;
     s.beta = p; p += d.K;
     s.W1b = reinterpret_cast<uint32_t*>(p); p += binary ? (size_t)d.Kw * d.Cout : 0;
+    s.W1z = reinterpret_cast<uint32_t*>(p); p += tern ? (size_t)d.Kw * d.Cout : 0;
     s.scale1 = p; p += d.Cout;
     s.a1 = p; p += d.Cout;
     s.c1 = p; p += d.Cout;
@@ -143,19 +148,20 @@ __device__ __forceinline__ float compute_q(const Smem& s, const Dims& d, int g, 
     return q;
 }
 
-template <bool BIN, int OPT>
-__global__ void __launch_bounds__(WARPS * 32, 3) svblock_edge_kernel(svnet_edge_params p)
+template <bool BIN, int OPT, bool TERN = false>
+__global__ void __launch_bounds__(WARPS * 32, 3) svblock_edge_kernel(svnet_edge_params p, const uint32_t* __restrict__ W1nz)
 {
     extern __shared__ __align__(16) float smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const Dims d = make_dims(p.in.Cs, p.in.Cv, p.k, p.Cout, p.Cvo, BIN);
-    const Smem s = carve(smem_raw, d, BIN, warp);
+    const Dims d = make_dims(p.in.Cs, p.in.Cv, p.k, p.Cout, p.Cvo, BIN, TERN);
+    const Smem s = carve(smem_raw, d, BIN, warp, TERN);
 
     // ---- CTA-shared parameters ----
     for (int i = threadIdx.x; i < 3 * d.Cve; i += blockDim.x) s.Wz[i] = p.Wz[i];
     if (BIN) {
         for (int i = threadIdx.x; i < d.K; i += blockDim.x) s.beta[i] = p.beta[i];
         for (int i = threadIdx.x; i < d.Kw * d.Cout; i += blockDim.x) s.W1b[i] = p.W1b[i];
+        if (TERN) for (int i = threadIdx.x; i < d.Kw * d.Cout; i += blockDim.x) s.W1z[i] = W1nz[i];
         for (int i = threadIdx.x; i < d.Cout; i += blockDim.x) s.scale1[i] = p.scale1[i];
     }
     for (int i = threadIdx.x; i < d.Cout; i += blockDim.x) { s.a1[i] = p.bn1_a[i]; s.c1[i] = p.bn1_c[i]; }
@@ -224,11 +230,12 @@ __global__ void __launch_bounds__(WARPS * 32, 3) svblock_edge_kernel(svnet_edge_
 #pragma unroll
                 for (int oo = 0; oo < OPT; ++oo) acc[e][oo] = 0;
             for (int wd = 0; wd < d.Kw; ++wd) {
-                uint32_t wv[OPT];
+                uint32_t wv[OPT], zv[OPT];
 #pragma unroll
                 for (int oo = 0; oo < OPT; ++oo) {
                     const int o = lane + 32 * oo;
                     wv[oo] = (o < d.Cout) ? s.W1b[wd * d.Cout + o] : 0u;
+                    zv[oo] = (TERN && o < d.Cout) ? s.W1z[wd * d.Cout + o] : 0u;
                 }
                 const uint32_t* Ap = s.A + wd * d.kp + eb;
                 const uint32_t* Mp = s.M + wd * d.kp + eb;
@@ -236,7 +243,15 @@ __global__ void __launch_bounds__(WARPS * 32, 3) svblock_edge_kernel(svnet_edge_
                 for (int e = 0; e < EB; ++e) {
                     const uint32_t a = Ap[e], m = Mp[e];
 #pragma unroll
-                    for (int oo = 0; oo < OPT; ++oo) acc[e][oo] += __popc((a ^ wv[oo]) & m);
+                    for (int oo = 0; oo < OPT; ++oo) {
+                        if (TERN) {
+                            // the accumulator holds the dot product itself: the count is per (edge, channel)
+                            const uint32_t mz = m & zv[oo];
+                            acc[e][oo] += __popc(mz) - 2 * __popc((a ^ wv[oo]) & mz);
+                        } else {
+                            acc[e][oo] += __popc((a ^ wv[oo]) & m);
+                        }
+                    }
                 }
             }
 #pragma unroll
@@ -247,7 +262,7 @@ __global__ void __launch_bounds__(WARPS * 32, 3) svblock_edge_kernel(svnet_edge_
 #pragma unroll
                     for (int e = 0; e < EB; ++e) {
                         if (eb + e < p.k) {
-                            const int dot = s.nvalid[eb + e] - 2 * acc[e][oo];
+                            const int dot = TERN ? acc[e][oo] : s.nvalid[eb + e] - 2 * acc[e][oo];
                             float y = __fmul_rn((float)dot, sc);
                             y = __fadd_rn(__fmul_rn(y, a1), c1);
                             y = y > 0.0f ? y : __fmul_rn(0.2f, y);
@@ -352,10 +367,10 @@ __global__ void __launch_bounds__(WARPS * 32, 3) svblock_edge_kernel(svnet_edge_
     }
 }
 
-template <bool BIN>
-int launch_edge(const svnet_edge_params* p, cudaStream_t st)
+template <bool BIN, bool TERN = false>
+int launch_edge(const svnet_edge_params* p, cudaStream_t st, const uint32_t* W1nz = nullptr)
 {
-    const Dims d = make_dims(p->in.Cs, p->in.Cv, p->k, p->Cout, p->Cvo, BIN);
+    const Dims d = make_dims(p->in.Cs, p->in.Cv, p->k, p->Cout, p->Cvo, BIN, TERN);
     const size_t smem = sizeof(float) * (d.shared_floats + WARPS * d.warp_floats);
     SV_REQUIRE(smem <= 220 * 1024, "svnet_svblock_edge_fwd: shared memory %zu B too large (Cs=%d Cv=%d k=%d Cout=%d)", smem,
                d.Cs, d.Cv, d.k, d.Cout);
@@ -363,9 +378,9 @@ int launch_edge(const svnet_edge_params* p, cudaStream_t st)
     const int opt = (p->Cout + 31) / 32;
 #define LAUNCH(O)                                                                                               \
     do {                                                                                                        \
-        SV_CUDA(cudaFuncSetAttribute(svblock_edge_kernel<BIN, O>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                                     (int)smem));                                                               \
-        svblock_edge_kernel<BIN, O><<<grid, WARPS * 32, smem, st>>>(*p);                                        \
+        SV_CUDA(cudaFuncSetAttribute(svblock_edge_kernel<BIN, O, TERN>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                     (int)smem));                                                                     \
+        svblock_edge_kernel<BIN, O, TERN><<<grid, WARPS * 32, smem, st>>>(*p, W1nz);                                  \
     } while (0)
     if (opt == 1) LAUNCH(1);
     else if (opt == 2) LAUNCH(2);
@@ -378,9 +393,10 @@ int launch_edge(const svnet_edge_params* p, cudaStream_t st)
 
 }  // namespace
 
-extern "C" int svnet_svblock_edge_fwd(const svnet_edge_params* p, void* stream)
+extern "C" int svnet_svblock_edge_fwd_nz(const svnet_edge_params* p, const uint32_t* W1nz, void* stream)
 {
     SV_REQUIRE(p, "svnet_svblock_edge_fwd: null params");
+    SV_REQUIRE(!W1nz || p->binary, "svnet_svblock_edge_fwd_nz: a non-zero plane needs a binary layer");
     SV_REQUIRE(p->in.s && p->in.v && p->idx && p->Wz && p->bn1_a && p->bn1_c && (p->PQ || (p->tab4 && p->W1tc)) && p->bn2_a &&
                    p->bn2_c && p->gate && p->out.s && p->out.v,
                "svnet_svblock_edge_fwd: null pointer");
@@ -399,11 +415,15 @@ extern "C" int svnet_svblock_edge_fwd(const svnet_edge_params* p, void* stream)
             if (h < 0) return h;
             if (h == 1) return SVNET_OK;
             SV_REQUIRE(p->PQ, "svnet_svblock_edge_fwd: layer not covered by the tensor-core kernel and no PQ table given");
-            h = svnet_edge_fast_dispatch(p, sv_stream(stream));
-            if (h < 0) return h;
-            if (h == 1) return SVNET_OK;
+            // the shape-specialised CUDA-core kernels assume +-1 weights: a layer with a non-zero plane takes the generic one
+            if (!W1nz) {
+                h = svnet_edge_fast_dispatch(p, sv_stream(stream));
+                if (h < 0) return h;
+                if (h == 1) return SVNET_OK;
+            }
         }
         SV_REQUIRE(p->PQ, "svnet_svblock_edge_fwd: the generic kernel needs the PQ table");
+        if (W1nz) return launch_edge<true, true>(p, sv_stream(stream), W1nz);
         return launch_edge<true>(p, sv_stream(stream));
     }
     SV_REQUIRE(p->Yab, "svnet_svblock_edge_fwd: fp layer needs Yab");
@@ -426,4 +446,9 @@ extern "C" int svnet_svblock_edge_fwd(const svnet_edge_params* p, void* stream)
         }
     }
     return launch_edge<false>(p, sv_stream(stream));
+}
+
+extern "C" int svnet_svblock_edge_fwd(const svnet_edge_params* p, void* stream)
+{
+    return svnet_svblock_edge_fwd_nz(p, nullptr, stream);
 }

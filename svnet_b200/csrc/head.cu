@@ -34,10 +34,18 @@ __device__ __forceinline__ float warp_sum(float v)
     return v;
 }
 
+// non-zero planes of ternary weights, one per layer (NULL: +-1)
+struct head_nz {
+    const uint32_t* z[3];
+};
+
 // prefetch != 0: the sign planes W1b of all binary layers (up to ~150 KB) are fetched into shared memory by cp.async.bulk
 // while the input row is loaded and sign-packed (round 2: the popcount loop's dependent-latency weight loads were 40 % of
 // the kernel's 31 us, the other threads' barrier waits another 30 %)
-__global__ void __launch_bounds__(NT) head_kernel(svnet_head_params p, int prefetch)
+// TERN: layers with a non-zero plane (nz.z[l]) count popc(m & z) - 2 popc((a ^ w) & m & z) per word; such calls do not
+// prefetch (the cls head's planes, 147 KB, would fill the prefetch area), so those layers read both planes with __ldg
+template <bool TERN>
+__global__ void __launch_bounds__(NT) head_kernel(svnet_head_params p, int prefetch, head_nz nz)
 {
     extern __shared__ __align__(16) float sm[];
     // two ping-pong activation buffers + sign words
@@ -118,7 +126,21 @@ __global__ void __launch_bounds__(NT) head_kernel(svnet_head_params p, int prefe
             }
             const uint32_t* wsm = wpre + pre_off;
             pre_off += (uint32_t)Kw * Cout;
+            const uint32_t* Z = TERN ? nz.z[l] : nullptr;
             for (int o = tid; o < Cout; o += NT) {
+                if (TERN && Z) {
+                    int dot = 0;
+#pragma unroll 16
+                    for (int w = 0; w < Kw; ++w) {
+                        const uint32_t mz = mask[w] & __ldg(Z + (long)w * Cout + o);
+                        dot += __popc(mz) - 2 * __popc((bits[w] ^ __ldg(L.W1b + (long)w * Cout + o)) & mz);
+                    }
+                    float y = __fmul_rn((float)dot, L.scale ? L.scale[o] : 1.0f);
+                    if (L.bias) y = __fadd_rn(y, L.bias[o]);
+                    if (L.bn_a) y = __fadd_rn(__fmul_rn(y, L.bn_a[o]), L.bn_c[o]);
+                    nxt[o] = sv_act(y, L.act);
+                    continue;
+                }
                 int mism = 0;
                 if (prefetch) {
 #pragma unroll 8
@@ -181,7 +203,7 @@ __global__ void __launch_bounds__(NT) head_kernel(svnet_head_params p, int prefe
 
 }  // namespace
 
-extern "C" int svnet_head_fwd(const svnet_head_params* p, void* stream)
+extern "C" int svnet_head_fwd_nz(const svnet_head_params* p, const uint32_t* const W1nz[3], void* stream)
 {
     SV_REQUIRE(p && p->x && p->out, "svnet_head_fwd: null pointer");
     SV_REQUIRE(p->nlayers >= 1 && p->nlayers <= 3 && p->K0 >= 1 && p->B >= 0, "svnet_head_fwd: bad shape");
@@ -215,10 +237,28 @@ extern "C" int svnet_head_fwd(const svnet_head_params* p, void* stream)
             Kl = L.Cout;
         }
     }
+    head_nz nz = {};
+    bool tern = false;
+    for (int l = 0; l < p->nlayers && W1nz; ++l) {
+        SV_REQUIRE(!W1nz[l] || p->layer[l].W1b, "svnet_head_fwd_nz: layer %d has a non-zero plane but no W1b", l);
+        nz.z[l] = W1nz[l];
+        tern = tern || W1nz[l] != nullptr;
+    }
+    if (tern) {
+        if (smem > 48 * 1024) SV_CUDA(cudaFuncSetAttribute(head_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        head_kernel<true><<<p->B, NT, smem, sv_stream(stream)>>>(*p, 0, nz);
+        SV_CHECK_LAUNCH("svnet_head_fwd_nz");
+        return SVNET_OK;
+    }
     const int prefetch = (pre > 0 && pre_ok && (smem & 15) == 0 && smem + pre <= 220 * 1024) ? 1 : 0;
     if (prefetch) smem += pre;
-    if (smem > 48 * 1024) SV_CUDA(cudaFuncSetAttribute(head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    head_kernel<<<p->B, NT, smem, sv_stream(stream)>>>(*p, prefetch);
+    if (smem > 48 * 1024) SV_CUDA(cudaFuncSetAttribute(head_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    head_kernel<false><<<p->B, NT, smem, sv_stream(stream)>>>(*p, prefetch, nz);
     SV_CHECK_LAUNCH("svnet_head_fwd");
     return SVNET_OK;
+}
+
+extern "C" int svnet_head_fwd(const svnet_head_params* p, void* stream)
+{
+    return svnet_head_fwd_nz(p, nullptr, stream);
 }

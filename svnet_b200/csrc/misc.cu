@@ -20,9 +20,11 @@ extern "C" const char* svnet_last_error(void) { return g_err; }
 
 namespace {
 
-// one warp per (row, word): lane = bit
+// one warp per (row, word): lane = bit.  NZ: also the non-zero plane (bit set = W != 0; -0.0 is zero as for torch.sign,
+// subnormals are not flushed: the library is built without -ftz)
+template <bool NZ>
 __global__ void pack_sign_kernel(const float* __restrict__ W, int rows, int K, int ldw, uint32_t* __restrict__ bits_t,
-                                 int* __restrict__ zero_count)
+                                 uint32_t* __restrict__ nz_t, int* __restrict__ zero_count)
 {
     const int Kw = (K + 31) / 32;
     const long gw = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -33,8 +35,11 @@ __global__ void pack_sign_kernel(const float* __restrict__ W, int rows, int K, i
     float v = (c < K) ? W[(long)row * ldw + c] : 0.0f;
     unsigned m = __ballot_sync(SV_FULL, v > 0.0f);
     unsigned z = __ballot_sync(SV_FULL, (c < K) && (v == 0.0f));
+    unsigned nz = 0;
+    if (NZ) nz = __ballot_sync(SV_FULL, (c < K) && (v != 0.0f));
     if (lane == 0) {
         bits_t[(long)w * rows + row] = m;
+        if (NZ) nz_t[(long)w * rows + row] = nz;
         if (z && zero_count) atomicAdd(zero_count, __popc(z));
     }
 }
@@ -165,8 +170,21 @@ extern "C" int svnet_pack_sign(const float* W, int rows, int K, int ldw, uint32_
     cudaStream_t st = sv_stream(stream);
     if (zero_count) SV_CUDA(cudaMemsetAsync(zero_count, 0, sizeof(int), st));
     const long warps = (long)rows * ((K + 31) / 32);
-    pack_sign_kernel<<<sv_cdiv(warps * 32, 256), 256, 0, st>>>(W, rows, K, ldw, bits_t, zero_count);
+    pack_sign_kernel<false><<<sv_cdiv(warps * 32, 256), 256, 0, st>>>(W, rows, K, ldw, bits_t, nullptr, zero_count);
     SV_CHECK_LAUNCH("svnet_pack_sign");
+    return SVNET_OK;
+}
+
+extern "C" int svnet_pack_sign_nz(const float* W, int rows, int K, int ldw, uint32_t* bits_t, uint32_t* nz_t, int* zero_count,
+                                  void* stream)
+{
+    SV_REQUIRE(W && bits_t && nz_t, "svnet_pack_sign_nz: null pointer");
+    SV_REQUIRE(rows >= 1 && K >= 1 && ldw >= K, "svnet_pack_sign_nz: bad shape rows=%d K=%d ldw=%d", rows, K, ldw);
+    cudaStream_t st = sv_stream(stream);
+    if (zero_count) SV_CUDA(cudaMemsetAsync(zero_count, 0, sizeof(int), st));
+    const long warps = (long)rows * ((K + 31) / 32);
+    pack_sign_kernel<true><<<sv_cdiv(warps * 32, 256), 256, 0, st>>>(W, rows, K, ldw, bits_t, nz_t, zero_count);
+    SV_CHECK_LAUNCH("svnet_pack_sign_nz");
     return SVNET_OK;
 }
 

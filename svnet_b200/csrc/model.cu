@@ -1,7 +1,9 @@
 // Whole-model C entry (SURVEY 8(b): svnet_model_create / _forward / _destroy): the SV-DGCNN classifier, binary or full precision,
 // (reference models/sv_dgcnn_cls.py:22-82) from a checkpoint's state_dict tensors to logits, without Python in the loop.
 //   create  : copies the tensors it needs, packs them once (sign bit-planes, folded BatchNorm affines, fp8 operand bytes of
-//             the tensor-core edge kernel, per-point table weights) -- the handle owns everything it uses afterwards;
+//             the tensor-core edge kernel, per-point table weights) -- the handle owns everything it uses afterwards.  A
+//             binarised weight slice with exact zeros (sign(0) = 0, sv_layers.py:45) keeps its non-zero plane as well and
+//             its layers take the *_nz entry points with it; zero-free slices keep none (the +-1 kernels);
 //   forward : sequences this library's own entry points with caller-owned scratch (svnet_model_workspace_bytes): no
 //             allocation, no host synchronisation -- capturable into a CUDA graph.  Launch structure as the Python path's: a
 //             batch of >= 32 768 points runs as two to four sub-batches (>= 16 384 points each) on the handle's streams, and inside each the chains that
@@ -35,18 +37,19 @@ struct svnet_model {
         int Cs, Cv, Cout, Cvo, H;      // Cs / Cv: per-point input dims (edge layers: half of the block's in_dims)
         float *G1, *G2, *Wz, *zscale, *W1, *beta, *scale1, *bn1_a, *bn1_c, *W2, *scale2, *bn2_a, *bn2_c;
         uint32_t* W1b;
+        uint32_t* W1nz;                // non-zero plane of linear1's weight, NULL when it has no exact zero
         unsigned char* W1tc;
         float *Wt, *cst, *Wab;        // Wab: [W1a; W1b] (2 Cout x Cs) of a full-precision linear1 (the Ya | Yb table)
         int NC;
     } conv[6];
     float *fuse_Wz, *fuse_zs;
     // head
-    uint32_t *h1_bits, *h2_bits;
+    uint32_t *h1_bits, *h2_bits, *h1_nz, *h2_nz;
     float *h1_beta, *h1_scale, *h1_a, *h1_c, *h2_beta, *h2_scale, *h2_a, *h2_c, *h3_W, *h3_b;
     float *h1_W, *h2_W;              // full-precision head
     // part segmentation: svfuse1 / 2 / 3, conv7 (labels), conv8 .. conv11
     float *f1_Wz, *f1_zs, *f2_Wz, *f2_zs, *f3_Wz, *f3_zs, *c7_W, *c7_a, *c7_c;
-    struct SegConv { float *beta, *scale, *bn_a, *bn_c; uint32_t *bits, *bits_c; float* W; int Cin, Cout; } c8, c9, c10;   // W: fp
+    struct SegConv { float *beta, *scale, *bn_a, *bn_c; uint32_t *bits, *bits_c, *nz, *nz_c; float* W; int Cin, Cout; } c8, c9, c10;   // W: fp
     float* c11_W;
     int C6s, C6v, Kc;
     // launch structure of svnet_model_forward: two sub-batch streams, each with an auxiliary stream for the chains that do
@@ -128,15 +131,26 @@ struct Loader {
         if (w && b && mu && var && *a && *c && svnet_fold_bn(w->data, b->data, mu->data, var->data, 1e-5f, C, *a, *c, st) != SVNET_OK)
             fail("svnet_fold_bn failed");
     }
-    // sign bit-planes [ceil(K/32)][rows]; the zero weights of call i are counted into zc[i] (device; svnet_pack_sign
-    // resets its counter)
+    // sign and non-zero bit-planes [ceil(K/32)][rows] of W [rows][ldw]; the zero weights of call i are counted into zc[i]
+    // (device; svnet_pack_sign_nz resets its counter).  *nzp receives the non-zero plane; once the counts are read back,
+    // drop_zero_free_planes() sets it to NULL where the slice holds no zero.
     int nz = 0;
-    uint32_t* bits(const float* W, int rows, int K, int* zc)
+    uint32_t** nz_slot[16] = {};
+    uint32_t* bits(const float* W, int rows, int K, int ldw, int* zc, uint32_t** nzp)
     {
-        uint32_t* d = static_cast<uint32_t*>(alloc(sizeof(uint32_t) * (size_t)((K + 31) / 32) * rows));
-        if (W && d && nz < 16 && svnet_pack_sign(W, rows, K, K, d, zc + nz, st) != SVNET_OK) fail("svnet_pack_sign failed");
+        const size_t bytes = sizeof(uint32_t) * (size_t)((K + 31) / 32) * rows;
+        uint32_t* d = static_cast<uint32_t*>(alloc(bytes));
+        *nzp = static_cast<uint32_t*>(alloc(bytes));
+        if (nz >= 16) fail("too many binarised weights");
+        else if (W && d && *nzp && svnet_pack_sign_nz(W, rows, K, ldw, d, *nzp, zc + nz, st) != SVNET_OK) fail("svnet_pack_sign_nz failed");
+        else nz_slot[nz] = nzp;
         ++nz;
         return d;
+    }
+    void drop_zero_free_planes(const int* zh)
+    {
+        for (int i = 0; i < nz && i < 16; ++i)
+            if (nz_slot[i] && zh[i] == 0) *nz_slot[i] = nullptr;
     }
 };
 
@@ -334,7 +348,7 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
         b.beta = L.dup(p + "linear1.beta", K1);
         b.scale1 = L.dup(p + "linear1.scale", b.Cout);
         b.scale2 = L.dup(p + "linear2.scale", b.Cvo);
-        b.W1b = L.bits(b.W1, b.Cout, K1, zc);
+        b.W1b = L.bits(b.W1, b.Cout, K1, K1, zc, &b.W1nz);
         if (l < 4) {
             const size_t wb = svnet_edge_tc_weight_bytes(b.Cs, b.Cv, b.Cout, b.Cvo, k);
             if (wb == 0) { L.fail(p + ": shape not covered by the tensor-core edge kernel"); break; }
@@ -386,7 +400,7 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
             const std::string p = std::string(name) + ".";
             c->Cin = Cin; c->Cout = Cout;
             c->beta = c->scale = c->W = nullptr;
-            c->bits = c->bits_c = nullptr;
+            c->bits = c->bits_c = c->nz = c->nz_c = nullptr;
             if (!binary) {     // full precision: the weight [Cout][Cin] as it is and the folded BN
                 c->W = L.dup(p + "0.weight", (long)Cout * Cin);
                 L.fold(p + "1", Cout, &c->bn_a, &c->bn_c);
@@ -399,15 +413,10 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
             if (!w) return;
             if (split > 0) {
                 // sign planes of the per-cloud columns [:, :split] and of the per-point columns [:, split:]
-                c->bits_c = static_cast<uint32_t*>(L.alloc(sizeof(uint32_t) * (size_t)((split + 31) / 32) * Cout));
-                c->bits = static_cast<uint32_t*>(L.alloc(sizeof(uint32_t) * (size_t)((Cin - split + 31) / 32) * Cout));
-                if (c->bits_c && c->bits && L.nz + 2 <= 16) {
-                    if (svnet_pack_sign(w->data, Cout, split, Cin, c->bits_c, zc + L.nz, L.st) != SVNET_OK) L.fail("svnet_pack_sign failed");
-                    if (svnet_pack_sign(w->data + split, Cout, Cin - split, Cin, c->bits, zc + L.nz + 1, L.st) != SVNET_OK) L.fail("svnet_pack_sign failed");
-                }
-                L.nz += 2;
+                c->bits_c = L.bits(w->data, Cout, split, Cin, zc, &c->nz_c);
+                c->bits = L.bits(w->data + split, Cout, Cin - split, Cin, zc, &c->nz);
             } else {
-                c->bits = L.bits(w->data, Cout, Cin, zc);
+                c->bits = L.bits(w->data, Cout, Cin, Cin, zc, &c->nz);
             }
         };
         seg_conv("conv8", m->Kc + Kp, 256, &m->c8, m->Kc);
@@ -429,8 +438,8 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
         m->fuse_zs = L.dup("svfuse.v2s.linear.scale", 3);
         const svnet_tensor* w1 = L.find("linear1.weight", (long)m->h1 * 2 * m->Cf);
         const svnet_tensor* w2 = L.find("linear2.weight", (long)m->h2 * m->h1);
-        m->h1_bits = L.bits(w1 ? w1->data : nullptr, m->h1, 2 * m->Cf, zc);
-        m->h2_bits = L.bits(w2 ? w2->data : nullptr, m->h2, m->h1, zc);
+        m->h1_bits = L.bits(w1 ? w1->data : nullptr, m->h1, 2 * m->Cf, 2 * m->Cf, zc, &m->h1_nz);
+        m->h2_bits = L.bits(w2 ? w2->data : nullptr, m->h2, m->h1, m->h1, zc, &m->h2_nz);
         m->h1_beta = L.dup("linear1.beta", 2 * m->Cf);
         m->h1_scale = L.dup("linear1.scale", m->h1);
         m->h2_beta = L.dup("linear2.beta", m->h1);
@@ -441,13 +450,12 @@ extern "C" int svnet_model_create(const char* kind, int k, int binary, int num_c
         m->h3_b = L.dup("linear3.bias", num_class);
     }
     if (L.ok) {
+        // zero counts per packed slice: keep a non-zero plane only where the slice has an exact zero
         int zh[16] = {0};
-        int zeros = 0;
         if (cudaMemcpyAsync(zh, zc, sizeof(zh), cudaMemcpyDeviceToHost, L.st) != cudaSuccess || cudaStreamSynchronize(L.st) != cudaSuccess)
             L.fail("CUDA error while packing");
-        for (int i = 0; i < 16; ++i) zeros += zh[i];
-        if (L.ok && zeros != 0)
-            L.fail("a binarised weight contains exact zeros (sign(0) = 0 plane not supported by the popcount kernels)");
+        else
+            L.drop_zero_free_planes(zh);
     }
     if (!L.ok) {
         svnet_set_error("svnet_model_create: %s", L.err.c_str());
@@ -581,7 +589,7 @@ int run_trunk(const svnet_model* m, const float* x, int B, int N, unsigned char*
             p.bn1_a = b.bn1_a; p.bn1_c = b.bn1_c; p.Cout = b.Cout;
             p.bn2_a = b.bn2_a; p.bn2_c = b.bn2_c; p.gate = gate; p.Cvo = b.Cvo; p.out = out;
             p.W1tc = b.W1tc; p.tab4 = table;
-            rc = svnet_svblock_edge_fwd(&p, stream);
+            rc = svnet_svblock_edge_fwd_nz(&p, b.W1nz, stream);
             if (rc != SVNET_OK) return rc;
         }
         prev.s = out.s; prev.lds = out.lds; prev.Cs = out.Cs;
@@ -642,12 +650,12 @@ int forward_cls_one(const svnet_model* m, const float* x, int B, int N, float* l
     }
     if (!m->binary) {
     } else if (pl.blp_bytes) {
-        rc = svnet_binlinear_pool_ws(bits, mask, R, K5, c5.W1b, c5.Cout, c5.scale1, c5.bn1_a, c5.bn1_c, N, g, g + Cf, 2 * Cf,
+        rc = svnet_binlinear_pool_nz(bits, mask, R, K5, c5.W1b, c5.W1nz, c5.Cout, c5.scale1, c5.bn1_a, c5.bn1_c, N, g, g + Cf, 2 * Cf,
                                      ws + pl.blp, pl.blp_bytes, sst);
         if (rc != SVNET_OK) return rc;
     } else {
         float* s5 = reinterpret_cast<float*>(ws + pl.s5);
-        rc = svnet_binlinear_rows_ws(bits, mask, nvalid, R, K5, c5.W1b, c5.Cout, c5.scale1, nullptr, c5.bn1_a, c5.bn1_c, SVNET_ACT_LEAKY,
+        rc = svnet_binlinear_rows_nz(bits, mask, nvalid, R, K5, c5.W1b, c5.W1nz, c5.Cout, c5.scale1, nullptr, c5.bn1_a, c5.bn1_c, SVNET_ACT_LEAKY,
                                      nullptr, 1, s5, c5.Cout, nullptr, pl.bl_bytes ? ws + pl.blp : nullptr, pl.bl_bytes, sst);
         if (rc != SVNET_OK) return rc;
         rc = svnet_pool_rows(s5, c5.Cout, c5.Cout, B, N, g, g + Cf, 2 * Cf, sst);
@@ -700,7 +708,8 @@ int forward_cls_one(const svnet_model* m, const float* x, int B, int N, float* l
     h.layer[1].bn_a = m->h2_a; h.layer[1].bn_c = m->h2_c; h.layer[1].act = SVNET_ACT_LEAKY;
     h.layer[2].Cout = m->ncls; h.layer[2].W = m->h3_W; h.layer[2].bias = m->h3_b; h.layer[2].act = SVNET_ACT_NONE;
     h.out = logits; h.ldo = m->ncls;
-    return svnet_head_fwd(&h, stream);
+    const uint32_t* nz[3] = {m->h1_nz, m->h2_nz, nullptr};
+    return svnet_head_fwd_nz(&h, nz, stream);
 }
 
 }  // namespace
@@ -913,12 +922,12 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
         rc = svnet_rows_prep(&cat, R, c5.Wz, c5.zscale, nullptr, c5.beta, nullptr, 0, nullptr, bits5, mask5, nvalid5, sst);
         if (rc != SVNET_OK) return rc;
         if (pl.blp_bytes) {
-            rc = svnet_binlinear_pool_ws(bits5, mask5, R, Kp, c5.W1b, C5s, c5.scale1, c5.bn1_a, c5.bn1_c, N, glob, nullptr, Kc, ws + pl.blp,
+            rc = svnet_binlinear_pool_nz(bits5, mask5, R, Kp, c5.W1b, c5.W1nz, C5s, c5.scale1, c5.bn1_a, c5.bn1_c, N, glob, nullptr, Kc, ws + pl.blp,
                                          pl.blp_bytes, sst);
             if (rc != SVNET_OK) return rc;
         } else {
             float* s5 = reinterpret_cast<float*>(ws + pl.s5);
-            rc = svnet_binlinear_rows_ws(bits5, mask5, nvalid5, R, Kp, c5.W1b, C5s, c5.scale1, nullptr, c5.bn1_a, c5.bn1_c, SVNET_ACT_LEAKY,
+            rc = svnet_binlinear_rows_nz(bits5, mask5, nvalid5, R, Kp, c5.W1b, c5.W1nz, C5s, c5.scale1, nullptr, c5.bn1_a, c5.bn1_c, SVNET_ACT_LEAKY,
                                          nullptr, 1, s5, C5s, nullptr, pl.bl_bytes ? ws + pl.blp : nullptr, pl.bl_bytes, sst);
             if (rc != SVNET_OK) return rc;
             rc = svnet_pool_rows(s5, C5s, C5s, B, N, glob, nullptr, Kc, sst);
@@ -958,7 +967,7 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
     if (m->binary) {
         rc = svnet_rows_prep(&pv, B, c6.Wz, c6.zscale, nullptr, c6.beta, nullptr, 0, nullptr, bits6, mask6, nvalid6, stream);
         if (rc != SVNET_OK) return rc;
-        rc = svnet_binlinear_rows_ws(bits6, mask6, nvalid6, B, C3, c6.W1b, C6s, c6.scale1, nullptr, c6.bn1_a, c6.bn1_c, SVNET_ACT_LEAKY,
+        rc = svnet_binlinear_rows_nz(bits6, mask6, nvalid6, B, C3, c6.W1b, c6.W1nz, C6s, c6.scale1, nullptr, c6.bn1_a, c6.bn1_c, SVNET_ACT_LEAKY,
                                      nullptr, 1, glob + C3, Kc, nullptr, nullptr, 0, stream);
         if (rc != SVNET_OK) return rc;
     } else {
@@ -1011,7 +1020,7 @@ int forward_seg_one(const svnet_model* m, const float* x, const float* label_one
     }
     svnet_seg_head_params h = seg_head_params(m, B, N);
     h.glob = glob; h.bits8 = bits8; h.mask8 = mask8; h.nvalid8 = nvalid8; h.logits = logits;
-    return svnet_seg_head_fwd(&h, ws + pl.head, pl.head_bytes, stream);
+    return svnet_seg_head_fwd_nz(&h, m->c8.nz_c, m->c8.nz, m->c9.nz, m->c10.nz, ws + pl.head, pl.head_bytes, stream);
 }
 
 }  // namespace

@@ -184,14 +184,19 @@ __global__ void __launch_bounds__(PW * 32) rows_prep_staged_kernel(svnet_view in
 // 64 rows x 64 outputs per CTA, 4x4 per thread, 16 words per smem chunk.
 constexpr int BR = 64, BO = 64, WC = 16;
 
+// TERN: ternary weights, W1nz [Kw][Cout] = non-zero plane.  The count of non-zero products then depends on (row, channel):
+// each word adds popc(m & z) - 2 popc((a ^ w) & m & z) to the accumulator, which holds the dot product itself (one
+// accumulator per (row, channel), not a count next to a mismatch sum, so the 4x4 tile needs no more registers).
+template <bool TERN>
 __global__ void __launch_bounds__(256) binlinear_rows_kernel(
     const uint32_t* __restrict__ bits, const uint32_t* __restrict__ mask, const int32_t* __restrict__ nvalid, long rows,
     int Kw, const uint32_t* __restrict__ W1b, int Cout, const float* __restrict__ scale, const float* __restrict__ bias,
     const float* __restrict__ bn_a, const float* __restrict__ bn_c, int act, const int32_t* __restrict__ cloud_dot,
-    long rows_per_cloud, float* __restrict__ out, int ldo, int32_t* __restrict__ out_i32)
+    long rows_per_cloud, float* __restrict__ out, int ldo, int32_t* __restrict__ out_i32, const uint32_t* __restrict__ W1nz)
 {
     __shared__ uint32_t As[WC][BR + 1], Ms[WC][BR + 1];
     __shared__ __align__(16) uint32_t Ws[WC][BO];
+    __shared__ __align__(16) uint32_t Zs[TERN ? WC : 1][BO];
     const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
     const long r0 = (long)blockIdx.x * BR;
     const int o0 = blockIdx.y * BO;
@@ -217,17 +222,32 @@ __global__ void __launch_bounds__(256) binlinear_rows_kernel(
             const int ww = i >> 6, oo = i & 63;
             const int w = w0 + ww, o = o0 + oo;
             Ws[ww][oo] = (w < Kw && o < Cout) ? W1b[(long)w * Cout + o] : 0u;
+            if (TERN) Zs[ww][oo] = (w < Kw && o < Cout) ? W1nz[(long)w * Cout + o] : 0u;
         }
         __syncthreads();
         const int wn = min(WC, Kw - w0);
         for (int ww = 0; ww < wn; ++ww) {
             const uint4 wv4 = *reinterpret_cast<const uint4*>(&Ws[ww][tx * 4]);
             const uint32_t wv[4] = {wv4.x, wv4.y, wv4.z, wv4.w};
+            if (TERN) {
+                const uint4 zv4 = *reinterpret_cast<const uint4*>(&Zs[ww][tx * 4]);
+                const uint32_t zv[4] = {zv4.x, zv4.y, zv4.z, zv4.w};
 #pragma unroll
-            for (int a = 0; a < 4; ++a) {
-                const uint32_t av = As[ww][ty * 4 + a], mv = Ms[ww][ty * 4 + a];
+                for (int a = 0; a < 4; ++a) {
+                    const uint32_t av = As[ww][ty * 4 + a], mv = Ms[ww][ty * 4 + a];
 #pragma unroll
-                for (int c = 0; c < 4; ++c) acc[a][c] += __popc((av ^ wv[c]) & mv);
+                    for (int c = 0; c < 4; ++c) {
+                        const uint32_t mz = mv & zv[c];
+                        acc[a][c] += __popc(mz) - 2 * __popc((av ^ wv[c]) & mz);
+                    }
+                }
+            } else {
+#pragma unroll
+                for (int a = 0; a < 4; ++a) {
+                    const uint32_t av = As[ww][ty * 4 + a], mv = Ms[ww][ty * 4 + a];
+#pragma unroll
+                    for (int c = 0; c < 4; ++c) acc[a][c] += __popc((av ^ wv[c]) & mv);
+                }
             }
         }
     }
@@ -235,13 +255,13 @@ __global__ void __launch_bounds__(256) binlinear_rows_kernel(
     for (int a = 0; a < 4; ++a) {
         const long r = r0 + ty * 4 + a;
         if (r >= rows) continue;
-        const int nv = nvalid[r];
+        const int nv = TERN ? 0 : nvalid[r];
         const long cb = cloud_dot ? (r / rows_per_cloud) * Cout : 0;
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
             const int o = o0 + tx * 4 + c;
             if (o >= Cout) continue;
-            int dot = nv - 2 * acc[a][c];
+            int dot = TERN ? acc[a][c] : nv - 2 * acc[a][c];
             if (cloud_dot) dot += cloud_dot[cb + o];
             if (out_i32) { out_i32[r * Cout + o] = dot; continue; }
             float y = __fmul_rn((float)dot, scale ? scale[o] : 1.0f);
@@ -290,16 +310,16 @@ extern "C" int svnet_rows_prep(const svnet_view* in, long rows, const float* Wz,
     return SVNET_OK;
 }
 
-int svnet_binlinear_tc_dispatch(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b, int Cout,
-                                const float* scale, const float* bias, const float* bn_a, const float* bn_c, int act,
-                                const int32_t* cloud_dot, long rows_per_cloud, float* out, int ldo, int32_t* out_i32,
-                                void* workspace, size_t workspace_bytes, cudaStream_t st);
+int svnet_binlinear_tc_dispatch(const uint32_t* bits, const uint32_t* mask, long rows, int K, const uint32_t* W1b,
+                                const uint32_t* W1nz, int Cout, const float* scale, const float* bias, const float* bn_a,
+                                const float* bn_c, int act, const int32_t* cloud_dot, long rows_per_cloud, float* out, int ldo,
+                                int32_t* out_i32, void* workspace, size_t workspace_bytes, cudaStream_t st);
 
-extern "C" int svnet_binlinear_rows_ws(const uint32_t* bits, const uint32_t* mask, const int32_t* nvalid, long rows, int K,
-                                       const uint32_t* W1b, int Cout, const float* scale, const float* bias,
-                                       const float* bn_a, const float* bn_c, int act, const int32_t* cloud_dot,
-                                       long rows_per_cloud, float* out, int ldo, int32_t* out_i32, void* workspace,
-                                       size_t workspace_bytes, void* stream)
+extern "C" int svnet_binlinear_rows_nz(const uint32_t* bits, const uint32_t* mask, const int32_t* nvalid, long rows, int K,
+                                       const uint32_t* W1b, const uint32_t* W1nz, int Cout, const float* scale,
+                                       const float* bias, const float* bn_a, const float* bn_c, int act,
+                                       const int32_t* cloud_dot, long rows_per_cloud, float* out, int ldo, int32_t* out_i32,
+                                       void* workspace, size_t workspace_bytes, void* stream)
 {
     SV_REQUIRE(bits && mask && nvalid && W1b, "svnet_binlinear_rows: null pointer");
     SV_REQUIRE(out || out_i32, "svnet_binlinear_rows: no output buffer");
@@ -309,17 +329,32 @@ extern "C" int svnet_binlinear_rows_ws(const uint32_t* bits, const uint32_t* mas
     SV_REQUIRE(!cloud_dot || rows_per_cloud >= 1, "svnet_binlinear_rows: rows_per_cloud");
     if (rows == 0) return SVNET_OK;
     if (workspace) {   // exact bf16 tensor-core path (binlinear_tc.cu) for the shapes it covers
-        const int handled = svnet_binlinear_tc_dispatch(bits, mask, rows, K, W1b, Cout, scale, bias, bn_a, bn_c, act, cloud_dot,
+        const int handled = svnet_binlinear_tc_dispatch(bits, mask, rows, K, W1b, W1nz, Cout, scale, bias, bn_a, bn_c, act, cloud_dot,
                                                         rows_per_cloud, out, ldo, out_i32, workspace, workspace_bytes,
                                                         sv_stream(stream));
         if (handled != 0) return handled < 0 ? handled : SVNET_OK;
     }
     dim3 grid(sv_cdiv(rows, BR), sv_cdiv(Cout, BO));
-    binlinear_rows_kernel<<<grid, 256, 0, sv_stream(stream)>>>(bits, mask, nvalid, rows, (K + 31) / 32, W1b, Cout, scale,
-                                                               bias, bn_a, bn_c, act, cloud_dot, rows_per_cloud, out, ldo,
-                                                               out_i32);
+    if (W1nz)
+        binlinear_rows_kernel<true><<<grid, 256, 0, sv_stream(stream)>>>(bits, mask, nvalid, rows, (K + 31) / 32, W1b, Cout, scale,
+                                                                         bias, bn_a, bn_c, act, cloud_dot, rows_per_cloud, out, ldo,
+                                                                         out_i32, W1nz);
+    else
+        binlinear_rows_kernel<false><<<grid, 256, 0, sv_stream(stream)>>>(bits, mask, nvalid, rows, (K + 31) / 32, W1b, Cout, scale,
+                                                                          bias, bn_a, bn_c, act, cloud_dot, rows_per_cloud, out, ldo,
+                                                                          out_i32, nullptr);
     SV_CHECK_LAUNCH("svnet_binlinear_rows");
     return SVNET_OK;
+}
+
+extern "C" int svnet_binlinear_rows_ws(const uint32_t* bits, const uint32_t* mask, const int32_t* nvalid, long rows, int K,
+                                       const uint32_t* W1b, int Cout, const float* scale, const float* bias,
+                                       const float* bn_a, const float* bn_c, int act, const int32_t* cloud_dot,
+                                       long rows_per_cloud, float* out, int ldo, int32_t* out_i32, void* workspace,
+                                       size_t workspace_bytes, void* stream)
+{
+    return svnet_binlinear_rows_nz(bits, mask, nvalid, rows, K, W1b, nullptr, Cout, scale, bias, bn_a, bn_c, act, cloud_dot,
+                                   rows_per_cloud, out, ldo, out_i32, workspace, workspace_bytes, stream);
 }
 
 extern "C" int svnet_binlinear_rows(const uint32_t* bits, const uint32_t* mask, const int32_t* nvalid, long rows, int K,

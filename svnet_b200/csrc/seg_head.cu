@@ -106,7 +106,9 @@ extern "C" size_t svnet_seg_head_workspace_bytes(const svnet_seg_head_params* p)
     return pl.total;
 }
 
-extern "C" int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspace, size_t workspace_bytes, void* stream)
+extern "C" int svnet_seg_head_fwd_nz(const svnet_seg_head_params* p, const uint32_t* W8c_nz, const uint32_t* W8p_nz,
+                                     const uint32_t* W9_nz, const uint32_t* W10_nz, void* workspace, size_t workspace_bytes,
+                                     void* stream)
 {
     SV_REQUIRE(p && p->logits && p->glob && p->beta8 && p->W8c && p->W8p && p->beta9 && p->W9 && p->beta10 && p->W10 && p->W11,
                "svnet_seg_head_fwd: null pointer");
@@ -139,8 +141,8 @@ extern "C" int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspac
     gv.s = p->glob; gv.lds = p->ldg; gv.Cs = p->Kc;
     rc = svnet_rows_prep(&gv, p->B, nullptr, nullptr, nullptr, p->beta8, nullptr, 0, nullptr, cb, cm, cn, stream);
     if (rc != SVNET_OK) return rc;
-    rc = svnet_binlinear_rows(cb, cm, cn, p->B, p->Kc, p->W8c, p->C8, nullptr, nullptr, nullptr, nullptr, SVNET_ACT_NONE, nullptr, 1,
-                              nullptr, 0, cdot, stream);
+    rc = svnet_binlinear_rows_nz(cb, cm, cn, p->B, p->Kc, p->W8c, W8c_nz, p->C8, nullptr, nullptr, nullptr, nullptr, SVNET_ACT_NONE,
+                                 nullptr, 1, nullptr, 0, cdot, nullptr, 0, stream);
     if (rc != SVNET_OK) return rc;
     // ---- conv8: per-point sign words of svfuse1(s_cat, v_cat), binarised linear + per-cloud part ----
     const uint32_t* b8 = p->bits8;
@@ -151,7 +153,7 @@ extern "C" int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspac
         if (rc != SVNET_OK) return rc;
         b8 = bits; m8 = mask; n8 = nvalid;
     }
-    rc = svnet_binlinear_rows_ws(b8, m8, n8, R, Kp, p->W8p, p->C8, p->scale8, nullptr, p->bn8_a, p->bn8_c, SVNET_ACT_LEAKY, cdot, p->N,
+    rc = svnet_binlinear_rows_nz(b8, m8, n8, R, Kp, p->W8p, W8p_nz, p->C8, p->scale8, nullptr, p->bn8_a, p->bn8_c, SVNET_ACT_LEAKY, cdot, p->N,
                                  hA, p->C8, nullptr, blws, pl.blws_bytes, stream);
     if (rc != SVNET_OK) return rc;
     // ---- conv9, conv10 ----
@@ -159,13 +161,13 @@ extern "C" int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspac
     hv.s = hA; hv.lds = p->C8; hv.Cs = p->C8;
     rc = svnet_rows_prep(&hv, R, nullptr, nullptr, nullptr, p->beta9, nullptr, 0, nullptr, bits, mask, nvalid, stream);
     if (rc != SVNET_OK) return rc;
-    rc = svnet_binlinear_rows_ws(bits, mask, nvalid, R, p->C8, p->W9, p->C9, p->scale9, nullptr, p->bn9_a, p->bn9_c, SVNET_ACT_LEAKY,
+    rc = svnet_binlinear_rows_nz(bits, mask, nvalid, R, p->C8, p->W9, W9_nz, p->C9, p->scale9, nullptr, p->bn9_a, p->bn9_c, SVNET_ACT_LEAKY,
                                  nullptr, 1, hB, p->C9, nullptr, blws, pl.blws_bytes, stream);
     if (rc != SVNET_OK) return rc;
     hv.s = hB; hv.lds = p->C9; hv.Cs = p->C9;
     rc = svnet_rows_prep(&hv, R, nullptr, nullptr, nullptr, p->beta10, nullptr, 0, nullptr, bits, mask, nvalid, stream);
     if (rc != SVNET_OK) return rc;
-    rc = svnet_binlinear_rows_ws(bits, mask, nvalid, R, p->C9, p->W10, p->C10, p->scale10, nullptr, p->bn10_a, p->bn10_c,
+    rc = svnet_binlinear_rows_nz(bits, mask, nvalid, R, p->C9, p->W10, W10_nz, p->C10, p->scale10, nullptr, p->bn10_a, p->bn10_c,
                                  SVNET_ACT_LEAKY, nullptr, 1, hA, p->C10, nullptr, blws, pl.blws_bytes, stream);
     if (rc != SVNET_OK) return rc;
     // ---- conv11 (full precision) and the (B, N, parts) -> (B, parts, N) transpose ----
@@ -175,6 +177,11 @@ extern "C" int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspac
     seg_transpose_kernel<<<dim3(sv_cdiv(p->N, 32), sv_cdiv(p->parts, 32), p->B), 256, 0, sv_stream(stream)>>>(hB, p->parts, p->N, p->logits);
     SV_CHECK_LAUNCH("svnet_seg_head_fwd(transpose)");
     return SVNET_OK;
+}
+
+extern "C" int svnet_seg_head_fwd(const svnet_seg_head_params* p, void* workspace, size_t workspace_bytes, void* stream)
+{
+    return svnet_seg_head_fwd_nz(p, nullptr, nullptr, nullptr, nullptr, workspace, workspace_bytes, stream);
 }
 
 // ---- full-precision head ----------------------------------------------------------------------------------------------

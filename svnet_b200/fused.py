@@ -239,9 +239,11 @@ def sv_edge_layer(s_in, v_in, B, N, k, blk, s_out, v_out, idx32=None, taps=None)
     p.Wz = Wz.data_ptr()
     p.zscale = zs.data_ptr() if zs is not None else 0
     keep = [gate, table, Wz, zs, a1, c1, a2, c2]
+    W1nz = None
     if blk.binary:
         lin = blk.linear1
-        beta, W1b, sc = lin.beta_vec(), lin.sign_bits(), lin.scale_vec()
+        beta, sc = lin.beta_vec(), lin.scale_vec()
+        W1b, W1nz = lin.sign_planes()
         p.beta, p.W1b, p.scale1 = beta.data_ptr(), W1b.data_ptr(), sc.data_ptr()
         keep += [beta, W1b, sc]
         if use_tc:
@@ -267,7 +269,7 @@ def sv_edge_layer(s_in, v_in, B, N, k, blk, s_out, v_out, idx32=None, taps=None)
         taps["bits"] = torch.zeros((R * k, Kw), dtype=torch.int32, device=dev)
         taps["mask"] = torch.zeros((R * k, Kw), dtype=torch.int32, device=dev)
         p.dbg_bits, p.dbg_mask = taps["bits"].data_ptr(), taps["mask"].data_ptr()
-    nv.svblock_edge_fwd(p)
+    nv.svblock_edge_fwd(p, W1nz=W1nz)
     if taps is not None:
         taps["gate"] = gate
     return idx32

@@ -177,12 +177,13 @@ class SV_DGCNN_PSEG(_Cached, nn.Module):
                 c8, c9, c10 = self.conv8[0], self.conv9[0], self.conv10[0]
                 Kc = glob.shape[1]
                 W11 = self.conv11.weight.detach()[:, :, 0]
-                layers = [dict(beta=c8.beta_vec(), bits=(c8.sign_bits(0, Kc), c8.sign_bits(Kc, c8.in_channels)), scale=c8.scale_vec(),
+                layers = [dict(beta=c8.beta_vec(), bits=(c8.sign_bits(0, Kc), c8.sign_bits(Kc, c8.in_channels)),
+                               nz=(c8.nz_bits(0, Kc), c8.nz_bits(Kc, c8.in_channels)), scale=c8.scale_vec(),
                                bn=self.conv8.bn_folded(), Cout=c8.out_channels),
-                          dict(beta=c9.beta_vec(), bits=c9.sign_bits(), scale=c9.scale_vec(), bn=self.conv9.bn_folded(),
+                          dict(beta=c9.beta_vec(), bits=c9.sign_bits(), nz=c9.nz_bits(), scale=c9.scale_vec(), bn=self.conv9.bn_folded(),
                                Cout=c9.out_channels),
-                          dict(beta=c10.beta_vec(), bits=c10.sign_bits(), scale=c10.scale_vec(), bn=self.conv10.bn_folded(),
-                               Cout=c10.out_channels)]
+                          dict(beta=c10.beta_vec(), bits=c10.sign_bits(), nz=c10.nz_bits(), scale=c10.scale_vec(),
+                               bn=self.conv10.bn_folded(), Cout=c10.out_channels)]
                 return nv.seg_head_fwd(sv_in[0], B, N, sv_in[2], sv_in[3], glob, layers, W11 if W11.is_contiguous() else W11.contiguous(),
                                        sv_bits=sv_bits)
             h = self.conv8[0].forward_rows(None, bn=self.conv8.bn_folded(), act=nv.ACT_LEAKY, cloud=glob, rows_per_cloud=N,

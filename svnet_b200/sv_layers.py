@@ -144,8 +144,16 @@ class Linear(_Cached, nn.Linear):
             self.scale = nn.Parameter(torch.ones(1, out_channels) / math.sqrt(in_channels))
 
     # -- packed forms ---------------------------------------------------------------------------
+    def sign_planes(self):
+        """(sign plane, non-zero plane or None): the weight's torch.sign in {-1, 0, +1} (nv.pack_sign_nz)."""
+        return self._packed("bits", ("weight",), lambda: nv.pack_sign_nz(self.weight.detach()))
+
     def sign_bits(self):
-        return self._packed("bits", ("weight",), lambda: nv.pack_sign(self.weight.detach()))
+        return self.sign_planes()[0]
+
+    def nz_bits(self):
+        """Non-zero plane of the weight, None when it has no exact zero (the +-1 kernels run)."""
+        return self.sign_planes()[1]
 
     def scale_vec(self):
         return self._packed("scale", ("scale",), lambda: self.scale.detach().reshape(-1).contiguous())
@@ -167,7 +175,7 @@ class Linear(_Cached, nn.Linear):
                 raise NotImplementedError("Linear(ba=True, bw=False) has no scale in the reference either")
             bits, mask, nvalid = nv.rows_prep(nv.view_of(x2d, None), rows, beta=self.beta_vec(), want_bits=True)
             return nv.binlinear_rows(bits, mask, nvalid, K, self.sign_bits(), Cout, scale=self.scale_vec(), bias=bias,
-                                     bn=bn, act=act, out=out, ldo=ldo)
+                                     bn=bn, act=act, out=out, ldo=ldo, W1nz=self.nz_bits())
         if out is None:
             out = torch.empty((rows, Cout), dtype=torch.float32, device=x2d.device)
             ldo = Cout
@@ -196,9 +204,17 @@ class Conv1d(_Cached, nn.Conv1d):
     def weight2d(self):
         return self._packed("w2d", ("weight",), lambda: self.weight.detach()[:, :, 0].contiguous())
 
-    def sign_bits(self, lo=0, hi=None):
+    def sign_planes(self, lo=0, hi=None):
+        """(sign plane, non-zero plane or None) of the input channels [lo, hi) (nv.pack_sign_nz)."""
         return self._packed(("bits", lo, hi), ("weight",),
-                            lambda: nv.pack_sign(self.weight.detach()[:, lo:hi, 0].contiguous()))
+                            lambda: nv.pack_sign_nz(self.weight.detach()[:, lo:hi, 0].contiguous()))
+
+    def sign_bits(self, lo=0, hi=None):
+        return self.sign_planes(lo, hi)[0]
+
+    def nz_bits(self, lo=0, hi=None):
+        """Non-zero plane of the input channels [lo, hi), None when that slice has no exact zero."""
+        return self.sign_planes(lo, hi)[1]
 
     def scale_vec(self):
         return self._packed("scale", ("scale",), lambda: self.scale.detach().reshape(-1).contiguous())
@@ -234,7 +250,7 @@ class Conv1d(_Cached, nn.Conv1d):
             cdot = None
             if cloud is not None:
                 cb, cm, cn = nv.rows_prep(nv.view_of(cloud, None), cloud.shape[0], beta=beta[:Kc], want_bits=True)
-                cdot = nv.binlinear_rows(cb, cm, cn, Kc, self.sign_bits(0, Kc), Cout, out_i32=True)
+                cdot = nv.binlinear_rows(cb, cm, cn, Kc, self.sign_bits(0, Kc), Cout, out_i32=True, W1nz=self.nz_bits(0, Kc))
             if sv_bits is not None:
                 bits, mask, nvalid = sv_bits
             elif sv_in is not None:
@@ -242,7 +258,8 @@ class Conv1d(_Cached, nn.Conv1d):
             else:
                 bits, mask, nvalid = nv.rows_prep(nv.view_of(x2d, None), rows, beta=beta[Kc:], want_bits=True)
             return nv.binlinear_rows(bits, mask, nvalid, Kp, self.sign_bits(Kc, Kc + Kp), Cout, scale=self.scale_vec(),
-                                     bn=bn, act=act, cloud_dot=cdot, rows_per_cloud=rows_per_cloud)
+                                     bn=bn, act=act, cloud_dot=cdot, rows_per_cloud=rows_per_cloud,
+                                     W1nz=self.nz_bits(Kc, Kc + Kp))
         if cloud is not None:
             B = cloud.shape[0]
             x2d = torch.cat([cloud.unsqueeze(1).expand(B, rows_per_cloud, Kc).reshape(rows, Kc), x2d], dim=1)
@@ -460,16 +477,19 @@ class SVBlock(_Cached, nn.Module):
             aux = aux_stream(dev)
         cur = torch.cuda.current_stream()
         if self.binary:
-            beta1, sbits, sc1 = self.linear1.beta_vec(), self.linear1.sign_bits(), self.linear1.scale_vec()
+            beta1, sc1 = self.linear1.beta_vec(), self.linear1.scale_vec()
+            sbits, snz = self.linear1.sign_planes()
         if aux is not None:
             aux.wait_stream(cur)
         with torch.cuda.stream(aux if aux is not None else cur):
             if self.binary:
                 bits, mask, nvalid = nv.rows_prep(view, R, Wz=Wz, zscale=zs, beta=beta1, want_bits=True)
                 if fused_pool:
-                    nv.binlinear_pool(bits, mask, K, sbits, Cso, sc1, bn1, rows_per_cloud, s_pool[0], s_pool[1], s_pool[2])
+                    nv.binlinear_pool(bits, mask, K, sbits, Cso, sc1, bn1, rows_per_cloud, s_pool[0], s_pool[1], s_pool[2],
+                                      W1nz=snz)
                 else:
-                    nv.binlinear_rows(bits, mask, nvalid, K, sbits, Cso, scale=sc1, bn=bn1, act=nv.ACT_LEAKY, out=s_out, ldo=lds_out)
+                    nv.binlinear_rows(bits, mask, nvalid, K, sbits, Cso, scale=sc1, bn=bn1, act=nv.ACT_LEAKY, out=s_out, ldo=lds_out,
+                                      W1nz=snz)
             else:
                 u = torch.empty((R, K), dtype=torch.float32, device=dev)
                 nv.rows_prep(view, R, Wz=Wz, zscale=zs, u_out=u, ldu=K)
@@ -590,7 +610,7 @@ def head_layer(lin, bn=None, act=nv.ACT_NONE):
     d = {"Cout": lin.out_features, "bn": bn, "act": act,
          "bias": lin.bias.detach() if lin.bias is not None else None}
     if getattr(lin, "ba", False):
-        d.update(W1b=lin.sign_bits(), beta=lin.beta_vec(), scale=lin.scale_vec())
+        d.update(W1b=lin.sign_bits(), W1nz=lin.nz_bits(), beta=lin.beta_vec(), scale=lin.scale_vec())
     elif getattr(lin, "bw", False):
         d.update(W=lin.weight.detach(), sign_w=True, scale=lin.scale_vec())
     else:
